@@ -2,6 +2,7 @@
 """Benchmark of the per-voxel T2 fit: masked-voxel fits per second (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--config c1|c2|c3|c4|c5] [--solver auto|fast|lbfgsb|lbfgsb_dense] [--impl reference]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 --config (default c2 = BASELINE.json configs[1], the configuration the metric is quoted on; the other four are the remaining
@@ -17,8 +18,12 @@ BASELINE configs, each with its own roofline / parity / cpu_baseline blocks, run
 
 One *pass* = the hot block of process_t2maps for one volume (run_t2mapping.py:411-461): zero the four dense maps, fit every
 masked voxel, residual epilogue, scatter into the dense maps, flags / iteration counts / final errors per voxel.  One *step* =
-`passes_per_step` back-to-back passes (chosen so that the K timed steps last >= 0.5 s: a c2 pass is 67 us, and a timed region of
-20 x 67 us cannot be cross-checked against a wall clock).
+`passes_per_step` back-to-back passes (chosen so that one step lasts >= 30 ms whatever K is, so that the default 20 timed steps
+last >= 0.6 s: a c2 pass is 67 us, and a timed region of 20 x 67 us cannot be cross-checked against a wall clock).
+
+--dump-outputs DIR (volume configurations c1 / c2 / c3 on one GPU): after the timed steps, what the last pass handed its caller --
+the four dense maps and the per-voxel fun / nit / status -- at a fixed, seeded sample of the masked voxels, as DIR/<name>.npy
+(see dump_outputs).  The inputs are seeded, so two builds run with the same arguments can be compared array for array.
 
   value     N = 1: whole-job fits/s of the step above with the volume resident in HBM.
             N > 1: the PRODUCT's multi-GPU path -- ONE job of N volume-sized slabs, every rank holds only its slab, fits it
@@ -74,7 +79,8 @@ LB_WHAT = {"lbfgsb": "the reference's own optimiser, scipy's compact 2m x 2m for
 LB_KERNEL = {"lbfgsb": "lbfgsb_kernel<%s> (one thread per voxel, FP64, compact matrices in local memory)",
              "lbfgsb_dense": "lbfgsb_dense_kernel<%s> (one thread per voxel, FP64, dense n x n matrix, state in registers + 480 B of pairs)"}
 SCALE = float(os.environ.get("T2FIT_BENCH_SCALE", "1.0"))       # shrinks every spatial axis (smoke runs of the bench itself)
-MIN_TIMED_S = float(os.environ.get("T2FIT_BENCH_MIN_S", "0.6"))
+MIN_STEP_S = float(os.environ.get("T2FIT_BENCH_MIN_STEP_S", "0.03"))
+DUMP_SAMPLE = 1 << 20           # masked voxels written by --dump-outputs: 7 float32 + 1 float64 arrays of 2^20 = 36 MB
 
 
 def measured_peaks():
@@ -308,8 +314,9 @@ def time_steps(c, step, steps, passes, finish=None):
     return max_over_ranks(c, e0.elapsed_time(e1))[0]
 
 
-def pick_passes(c, step, steps, finish=None):
-    """passes per step so that the timed region lasts >= MIN_TIMED_S (same on every rank)."""
+def pick_passes(c, step, finish=None):
+    """passes per step so that one step lasts >= MIN_STEP_S (same on every rank); independent of the step count, so that
+    --steps K times K steps of the same size."""
     torch = c.torch
     for _ in range(3):
         step()
@@ -326,7 +333,7 @@ def pick_passes(c, step, steps, finish=None):
     e1.record(c.stream)
     torch.cuda.synchronize()
     per = max_over_ranks(c, e0.elapsed_time(e1) / n)[0] * 1e-3
-    return int(np.clip(np.ceil(MIN_TIMED_S / (steps * max(per, 1e-7))), 1, 5000))
+    return int(np.clip(np.ceil(MIN_STEP_S / max(per, 1e-7)), 1, 5000))
 
 
 def slab_hashes(torch, fields, bounds):
@@ -340,6 +347,23 @@ def slab_hashes(torch, fields, bounds):
             row.append(v.view(torch.int32).to(torch.int64).sum() if v.dtype == torch.float32 else v.to(torch.int64).sum())
         rows.append(torch.stack(row))
     return torch.stack(rows)
+
+
+def dump_outputs(torch, out_dir, maps, idx_d, per_voxel):
+    """--dump-outputs: the dense maps (t2, k, sigma, res) and the per-voxel outputs (fun, nit, status) of the last pass at a
+    fixed, seeded sample of DUMP_SAMPLE masked voxels (all of them if there are fewer), as float32 .npy files;
+    voxel_index.npy (float64, exact) holds each sampled voxel's flat index in the volume.  Off-mask voxels are left out:
+    the bench asserts that they are zero."""
+    m = idx_d.numel()
+    pick = np.arange(m) if m <= DUMP_SAMPLE else np.sort(np.random.default_rng(0).choice(m, DUMP_SAMPLE, replace=False))
+    pick_d = torch.from_numpy(pick).to(idx_d.device)
+    vox_d = idx_d[pick_d]
+    arrays = {"voxel_index": vox_d.to(torch.float64)}
+    arrays.update({name: maps[i][vox_d] for i, name in enumerate(("t2", "k", "sigma", "res"))})
+    arrays.update({name: v[pick_d].to(torch.float32) for name, v in per_voxel.items()})
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.cpu().numpy())
 
 
 def parity_block(c, cfg, rows, te, oracle, solver):
@@ -573,7 +597,7 @@ def bench_volume(args, cfg):
     main_finish = (None if fa is not None else sharded_finish) if c.world > 1 else None
     for _ in range(max(3, args.warmup)):
         main_pass()
-    passes = pick_passes(c, main_pass, args.steps, main_finish)
+    passes = pick_passes(c, main_pass, main_finish)
     for _ in range(max(3, args.warmup)):                  # W warm-up STEPS of the final shape
         for _ in range(min(passes, 50)):
             main_pass()
@@ -581,6 +605,8 @@ def bench_volume(args, cfg):
         main_finish()
     elapsed_ms = time_steps(c, main_pass, args.steps, passes, main_finish)
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs:                                 # the maps still hold the last timed pass (one GPU: dense_pass)
+        dump_outputs(torch, args.dump_outputs, maps, idx_d, {"fun": fun_d, "nit": nit_d, "status": st_d})
     m_total = sum_over_ranks(c, m_s if c.world > 1 else m)
     value = m_total * args.steps * passes / (elapsed_ms * 1e-3)
     pass_ms = elapsed_ms / (args.steps * passes)
@@ -616,13 +642,13 @@ def bench_volume(args, cfg):
         ok_all = torch.tensor([int(ok_g and fit_ok and ok_fused is not False)], device=c.dev, dtype=torch.int32)
         c.dist.all_reduce(ok_all, op=c.dist.ReduceOp.MIN)
         assert int(ok_all[0]) == 1, "sharded fit + gather differs from the single-GPU fit"
-        p_fit = pick_passes(c, fit_only_pass, args.steps)
+        p_fit = pick_passes(c, fit_only_pass)
         fit_ms = time_steps(c, fit_only_pass, args.steps, p_fit) / (args.steps * p_fit)
-        p_one = pick_passes(c, single_job_pass, args.steps)
+        p_one = pick_passes(c, single_job_pass)
         one_ms = time_steps(c, single_job_pass, args.steps, p_one) / (args.steps * p_one)
-        p_pipe = pick_passes(c, sharded_pass, args.steps, sharded_finish)
+        p_pipe = pick_passes(c, sharded_pass, sharded_finish)
         pipe_ms = time_steps(c, sharded_pass, args.steps, p_pipe, sharded_finish) / (args.steps * p_pipe)
-        p_rep = pick_passes(c, dense_pass, args.steps)
+        p_rep = pick_passes(c, dense_pass)
         rep_ms = time_steps(c, dense_pass, args.steps, p_rep) / (args.steps * p_rep)
         bytes_in = sum((c.world - 1) * L * (1 if n == "status" else 4) for n in names)
         extra["sharded"] = {"form": "fused all-gather" if fa is not None else "NCCL all-gather, pipelined",
@@ -649,7 +675,7 @@ def bench_volume(args, cfg):
             okt = torch.tensor([int(ok2)], device=c.dev, dtype=torch.int32)
             c.dist.all_reduce(okt, op=c.dist.ReduceOp.MIN)
             assert int(okt[0]) == 1, "fused gather of T2 / S0 differs"
-            p2s = pick_passes(c, fused_pass_t2s0, args.steps)
+            p2s = pick_passes(c, fused_pass_t2s0)
             t2s0_ms = time_steps(c, fused_pass_t2s0, args.steps, p2s) / (args.steps * p2s)
             extra["sharded_t2_s0_only"] = {"value": m_total / (t2s0_ms * 1e-3), "ms_per_pass": t2s0_ms,
                                            "gather_bytes_received_per_rank": int((c.world - 1) * L * 8),
@@ -725,7 +751,7 @@ def bench_volume(args, cfg):
 
         def plain_pass():
             lib.t2fit_run(C.byref(p), C.byref(o_fit), c.stream.cuda_stream)
-        pp = pick_passes(c, plain_pass, args.steps)
+        pp = pick_passes(c, plain_pass)
         plain_ms = time_steps(c, plain_pass, max(3, args.steps // 4), pp) / (max(3, args.steps // 4) * pp)
         flops = float((wm["flop_fixed"] + wm["flop_per_pass"] * nit).sum())
         mufu = float((wm["mufu_fixed"] + wm["mufu_per_pass"] * nit).sum())
@@ -902,7 +928,7 @@ def bench_series(args, cfg):
 
         def dev_pass():
             c.lib.t2fit_run(C.byref(p), C.byref(o), c.stream.cuda_stream)
-        pp = pick_passes(c, dev_pass, args.steps)
+        pp = pick_passes(c, dev_pass)
         dev_ms = time_steps(c, dev_pass, 3, pp) / (3 * pp)
         mv = idx.numel()
         step_bytes = mv * (4.0 * n_echo + 8 + 12 + 1) + n_vox + 4.0 * (3 * (n_vox - mv) + n_vox)
@@ -1033,7 +1059,10 @@ def main():
     ap.add_argument("--no-cpu-baseline", dest="no_cpu_baseline", action="store_true")
     ap.add_argument("--no-secondary", dest="no_secondary", action="store_true")
     ap.add_argument("--no-lbfgsb", dest="no_secondary", action="store_true")      # round-1 name of --no-secondary
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed pass as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or CONFIGS[args.config]["kind"] != "volume" or args.gpus != 1):
+        ap.error("--dump-outputs is available for the volume configurations (c1, c2, c3) of the CUDA arm on one GPU")
     if args.impl == "reference":
         run_reference(args)
         return
