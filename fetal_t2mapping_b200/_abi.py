@@ -8,7 +8,7 @@ from __future__ import annotations
 import ctypes as C
 import os
 
-ABI_VERSION = 4
+ABI_VERSION = 5
 MAX_ECHO = 32
 MAX_DUP = 7
 
@@ -124,6 +124,8 @@ SYMBOLS = [
     ("t2fit_scatter", C.c_int, [C.POINTER(C.c_void_p), C.POINTER(C.c_void_p), C.c_int32, C.c_void_p, C.c_int64,
                                 C.c_void_p]),
     ("t2fit_residuals", C.c_int, [C.POINTER(Problem), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    ("t2fit_stderr", C.c_int, [C.POINTER(Problem), C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p,
+                               C.c_void_p, C.c_void_p]),
     ("t2fit_work_model", C.c_int, [C.c_int32, C.c_int32] + [C.POINTER(C.c_double)] * 5),
 ]
 

@@ -25,8 +25,8 @@ import numpy as np
 from . import _abi
 from .presets import NO_PRIOR_K_UB, NO_PRIOR_T2_BOUNDS
 
-__all__ = ["fit_voxels_batch", "fit_voxels_into", "check_counts", "t2map_volume", "compute_residuals", "FitResult", "init", "shutdown", "device_info",
-           "mask_indices_device", "work_model", "pinned_array", "BOUNDS_ERROR"]
+__all__ = ["fit_voxels_batch", "fit_voxels_into", "check_counts", "t2map_volume", "compute_residuals", "parameter_stderr", "FitResult", "init",
+           "shutdown", "device_info", "mask_indices_device", "work_model", "pinned_array", "BOUNDS_ERROR"]
 
 BOUNDS_ERROR = "An upper bound is less than the corresponding lower bound."   # scipy's text
 
@@ -136,6 +136,8 @@ class FitResult:
     ``status``             uint8[M]  0 ok / 1 non-finite input / 2 iteration cap / 3 bad bounds
     ``iteration_infos``    the callback traces (:180-234) when the call asked for them (``trace_cap``,
                            L-BFGS-B solver), else ``[]`` per voxel
+    ``se_k``, ``se_t2``, ``se_sigma``  f32[M] standard errors of the parameters (``want`` with "se"; see
+                           :func:`parameter_stderr`), else None; ``standard_errors`` stacks them as ``results`` does
     For device calls the float fields are torch CUDA tensors (float32).
     """
     t2: object
@@ -151,6 +153,9 @@ class FitResult:
     trace_f: object = None       # float32[M, trace_cap]  f_val per L-BFGS-B iteration
     trace_step: object = None    # float32[M, trace_cap]  step_size (NaN for the first iteration)
     trace_len: object = None     # int32[M]               entries used = min(nit, trace_cap)
+    se_k: object = None          # float32[M]             standard errors (want "se"); se_sigma None for gaussian
+    se_t2: object = None
+    se_sigma: object = None
 
     @property
     def sigma(self):
@@ -176,6 +181,17 @@ class FitResult:
     def results(self):
         cols = [self.k, self.t2] + ([self.sigma] if self.fit != "gaussian" else [])
         if _is_torch(self.k):
+            import torch
+            return torch.stack(cols, dim=1).double()
+        return np.stack(cols, axis=1).astype(np.float64)
+
+    @property
+    def standard_errors(self):
+        """f64[M,P] standard errors in the order of ``results`` (k, T2[, sigma]); None unless the call asked for "se"."""
+        if self.se_t2 is None:
+            return None
+        cols = [self.se_k, self.se_t2] + ([self.se_sigma] if self.fit != "gaussian" else [])
+        if _is_torch(self.se_t2):
             import torch
             return torch.stack(cols, dim=1).double()
         return np.stack(cols, axis=1).astype(np.float64)
@@ -284,6 +300,33 @@ def _run(lib, p, o, stream):
         raise _abi.T2FitError(f"t2fit_run: {_abi.ERRORS.get(rc, rc)}: {msg}")
 
 
+def _stderr_launch(lib, p, fit, params, dense, se, stream):
+    """t2fit_stderr on the echoes / indices / sizes already in ``p`` (device AoS): ``params`` (k, t2, sigma) and ``se``
+    (se_k, se_t2, se_sigma) are device addresses or None."""
+    k, t2, sg = params
+    _abi.check(lib, lib.t2fit_stderr(C.byref(p), k, t2, sg if fit != "gaussian" else None, int(dense), *se, stream),
+               "t2fit_stderr")
+
+
+def _stderr_staged(lib, p, fit, rows, k, t2, sigma):
+    """Standard errors of host rows ``rows`` [M, E] at compact host parameters: rows and parameters are staged to the
+    device through torch (as :func:`compute_residuals` does), the results copied back as float32 numpy [M] arrays."""
+    import torch
+    dev = torch.device("cuda", _state["device"])
+    m = rows.shape[0]
+    y = torch.from_numpy(np.ascontiguousarray(rows, dtype=np.float32)).to(dev)
+    par = [torch.from_numpy(np.ascontiguousarray(a, dtype=np.float32)).to(dev) if a is not None else None for a in (k, t2, sigma)]
+    out = torch.zeros((3, m), dtype=torch.float32, device=dev)
+    q = _abi.Problem.from_buffer_copy(p)
+    q.echoes, q.memory, q.layout, q.mask_idx, q.idx_dtype = y.data_ptr(), _abi.MEM_DEVICE, _abi.LAYOUT_AOS, None, _abi.IDX_I64
+    q.n_vox, q.n_fit, q.ld = m, m, 0
+    if m:
+        _stderr_launch(lib, q, fit, [t.data_ptr() if t is not None else None for t in par], 0,
+                       [out[i].data_ptr() for i in range(3)], torch.cuda.current_stream(dev).cuda_stream)
+    o = out.cpu().numpy()
+    return o[0], o[1], (o[2] if fit != "gaussian" else None)
+
+
 def fit_voxels_batch(reshaped_t2w, mask_indices, TEeffs, fit, fit_params, prior=True, norm=False, *,
                      solver="auto", trace_cap=0, max_iter=0, tol=0.0, init_mode="auto", check_bounds=True,
                      dense_out=None, want=("nit", "fun", "status")) -> FitResult:
@@ -297,6 +340,8 @@ def fit_voxels_batch(reshaped_t2w, mask_indices, TEeffs, fit, fit_params, prior=
     ``solver``: 'fast' | 'lbfgsb_dense' | 'lbfgsb' | 'auto' (see :func:`resolve_solver`).  ``trace_cap`` > 0 (L-BFGS-B solver)
     also returns the callback trace of every fitted voxel (``FitResult.iteration_infos``) -- meant for the
     sampled voxels of the convergence plots (utils/t2map_utils.py:115-292), pass their indices only.
+    ``want`` with "se": also the standard errors of the fitted parameters (``FitResult.se_*``, :func:`parameter_stderr`),
+    computed by a second kernel on the same stream from the compact results; asynchronous for device inputs.
     """
     lib = init()
     solver = resolve_solver(fit, solver)
@@ -376,6 +421,17 @@ def fit_voxels_batch(reshaped_t2w, mask_indices, TEeffs, fit, fit_params, prior=
     o.fun, o.nit, o.status = ptr(out["fun"]), ptr(out["nit"]), ptr(out["status"])
     o.dense = 0
     _run(lib, p, o, stream)
+    se = (None, None, None)
+    if "se" in want:
+        if dev:
+            se_t = torch.empty((3, m), dtype=torch.float32, device=y.device)
+            if m:
+                _stderr_launch(lib, p, fit, [ptr(out["k"]), ptr(out["t2"]), ptr(out["sigma"])], 0,
+                               [se_t[i].data_ptr() for i in range(3)], stream)
+            se = (se_t[0], se_t[1], se_t[2] if fit != "gaussian" else None)
+        else:
+            rows = y if idx is None else y[idx]
+            se = _stderr_staged(lib, p, fit, rows, out["k"], out["t2"], out["sigma"])
     if dev:
         counts = None
         if check_bounds:                           # one small D2H: waits for the call (check_bounds=False stays asynchronous)
@@ -389,7 +445,7 @@ def fit_voxels_batch(reshaped_t2w, mask_indices, TEeffs, fit, fit_params, prior=
             raise ValueError(BOUNDS_ERROR)
     return FitResult(out["t2"], out["k"], out["sigma"], out["res"], out["fun"], out["nit"], out["status"], fit,
                      counts if counts is not None else (0, 0, 0, 0), solver, out.get("trace_f"), out.get("trace_step"),
-                     out.get("trace_len"))
+                     out.get("trace_len"), *se)
 
 
 def fit_voxels_into(reshaped_t2w, mask_indices, TEeffs, fit, fit_params, prior, norm, out, *, solver="auto", counts=None):
@@ -456,10 +512,12 @@ def mask_indices_device(mask, n_masks=None):
     return idx[:n.value]
 
 
-def t2map_volume(t2w, mask, TEeffs, fit, fit_params, prior=True, norm=False, **kw):
+def t2map_volume(t2w, mask, TEeffs, fit, fit_params, prior=True, norm=False, stderr=False, **kw):
     """Stacked per-TE volumes ``t2w[z,y,x,E]``, mask ``[z,y,x]`` or per-TE masks ``[z,y,x,E]`` and the
     TE vector in; ``(t2_map, k_map, sigma_map, res_map)`` float32 ``[z,y,x]`` out, zeros off-mask --
-    the whole hot block of ``process_t2maps`` (run_t2mapping.py:383-386, :411-461, :471-473)."""
+    the whole hot block of ``process_t2maps`` (run_t2mapping.py:383-386, :411-461, :471-473).
+    ``stderr=True`` adds a fifth element ``(se_t2_map, se_k_map, se_sigma_map)``: the standard errors of the fitted
+    parameters (:func:`parameter_stderr`), float32 ``[z,y,x]``, zeros off-mask (se_sigma all zeros for 'gaussian')."""
     lib = init()
     shape3 = tuple(t2w.shape[:3])
     n_echo = t2w.shape[-1]
@@ -512,7 +570,20 @@ def t2map_volume(t2w, mask, TEeffs, fit, fit_params, prior=True, norm=False, **k
         _raise_for_counts([int(v) for v in dcnt.cpu()])
     elif o.status_count[3] > 0:
         raise ValueError(BOUNDS_ERROR)
-    return tuple(maps[i].reshape(shape3) for i in range(4))
+    out = tuple(maps[i].reshape(shape3) for i in range(4))
+    if not stderr:
+        return out
+    if stream is not None:
+        se = torch.zeros((3, n_vox), dtype=torch.float32, device=y.device)
+        if m:
+            _stderr_launch(lib, p, fit, [mp[1], mp[0], mp[2]], 1, [se[1].data_ptr(), se[0].data_ptr(), se[2].data_ptr()], stream)
+    else:
+        se = np.zeros((3, n_vox), np.float32)
+        sk, st, ss = _stderr_staged(lib, p, fit, y[idx], maps[1][idx], maps[0][idx], maps[2][idx])
+        se[0][idx], se[1][idx] = st, sk
+        if ss is not None:
+            se[2][idx] = ss
+    return out + (tuple(se[i].reshape(shape3) for i in range(3)),)
 
 
 def compute_residuals(reshaped_t2w, TEeffs, fit, norm, k_map, t2_map, sigma_map, res_map, mask_indices, mask):
@@ -545,3 +616,43 @@ def compute_residuals(reshaped_t2w, TEeffs, fit, norm, k_map, t2_map, sigma_map,
     if host:
         return res.cpu().numpy().reshape(shape3)
     return res.reshape(shape3)
+
+
+def parameter_stderr(reshaped_t2w, TEeffs, fit, norm, k_map, t2_map, sigma_map, mask_indices, mask):
+    """Standard errors of the fitted parameters for maps that already exist (e.g. read back from NIfTI), with the
+    argument conventions of :func:`compute_residuals`; returns ``(se_t2_map, se_k_map, se_sigma_map)`` float32 shaped like
+    ``mask``, zeros off-mask (se_sigma all zeros for 'gaussian').  Runs the CUDA pass ``t2fit_stderr``; numpy inputs are
+    staged through torch and numpy maps come back.
+
+    Per voxel, in FP64, at the given parameters theta = (k, T2[, sigma]) with bounds ignored: for 'gaussian' and
+    'gaussian_rician' ``sqrt(diag(s^2 (J'J)^-1))`` with ``s^2 = sum_e r_e^2 / (E - P)`` (scipy ``curve_fit``'s ``pcov``);
+    for 'rician' ``sqrt(diag(H^-1))``, H the Hessian of the summed negative log-likelihood.  NaN where the voxel's input
+    is not finite (rician: an echo <= 0), T2 <= 0, E <= P, or the matrix is not positive definite (DESIGN.md section 11)."""
+    import torch
+    lib = init()
+    dev = torch.device("cuda", _state["device"])
+    host = not _is_torch(reshaped_t2w)
+
+    def to_dev(a, dt):
+        t = a if _is_torch(a) else torch.from_numpy(np.ascontiguousarray(a))
+        return t.to(device=dev, dtype=dt).contiguous()
+    y = to_dev(reshaped_t2w, torch.float32)
+    idx = to_dev(mask_indices, torch.int64)
+    k, t2, sg = (to_dev(a, torch.float32).reshape(-1) for a in (k_map, t2_map, sigma_map))
+    se = torch.zeros((3, y.shape[0]), dtype=torch.float32, device=dev)
+    p = _abi.Problem()
+    dummy = {"initial_guess": [1.0, 100.0] + ([1.0] if fit != "gaussian" else []),
+             "param_bounds": [(0.0, 1e9), (1e-3, 1e9)] + ([(0.0, 1e9)] if fit != "gaussian" else [])}
+    keep = _fill_problem(p, fit, dummy, TEeffs, True, norm, 0, 0.0, "loglinear")
+    if y.dim() != 2 or y.shape[1] != p.n_echo:
+        raise ValueError(f"reshaped_t2w must be [N, {p.n_echo}]")
+    p.echoes, p.memory, p.layout, p.mask_idx = y.data_ptr(), _abi.MEM_DEVICE, _abi.LAYOUT_AOS, idx.data_ptr()
+    p.n_vox, p.n_fit = y.shape[0], idx.numel()
+    stream = torch.cuda.current_stream(dev).cuda_stream
+    _stderr_launch(lib, p, fit, [k.data_ptr(), t2.data_ptr(), sg.data_ptr()], 1,
+                   [se[1].data_ptr(), se[0].data_ptr(), se[2].data_ptr()], stream)
+    del keep
+    shape3 = tuple(mask.shape[:3])
+    if host:
+        se = se.cpu().numpy()
+    return tuple(se[i].reshape(shape3) for i in range(3))

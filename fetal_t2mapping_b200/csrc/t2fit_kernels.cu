@@ -40,6 +40,7 @@
 #include "t2fit_consts.h"
 #include "t2fit_lbfgsb_coop.cuh"
 #include "t2fit_lbfgsb_dense.cuh"
+#include "t2fit_stderr.cuh"
 #include "t2fit_workers.h"
 
 using namespace t2fit;
@@ -1012,6 +1013,70 @@ __global__ void __launch_bounds__(256) residual_kernel(const __grid_constant__ F
         acc += __ldg(p + e) * scale - pred;
     }
     res_map[row] = acc / (float)c.n_echo;
+}
+
+// ------------------------------------------------------------------------------------------------
+// stderr_kernel: per-voxel standard errors of (k, T2[, sigma]) at given parameters (t2fit_stderr, csrc/t2fit_stderr.cuh).
+// One thread per voxel, FP64; echoes read as the fit kernels read AoS rows (vector loads where E and the base allow).
+// ------------------------------------------------------------------------------------------------
+struct StderrArgs {
+    double te[kMaxEcho];
+    const float* echoes;
+    const int64_t* idx;        // at most one of idx / idx32 is set; neither = rows 0..n_fit-1
+    const int32_t* idx32;
+    int64_t n_fit, n_vox;
+    const float *k, *t2, *sigma;
+    float *se_k, *se_t2, *se_sigma;
+    int dense;                 // parameters and standard errors indexed by row instead of i
+    int norm;
+    int vec_ok;
+};
+
+template <int MODEL, int E>
+__global__ void __launch_bounds__(256) stderr_kernel(const __grid_constant__ StderrArgs a) {
+    const int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x;
+    if (i >= a.n_fit) return;
+    const int64_t row = a.idx ? __ldg(a.idx + i) : a.idx32 ? (int64_t)__ldg(a.idx32 + i) : i;
+    const bool in_range = (unsigned long long)row < (unsigned long long)a.n_vox;
+    const int64_t o = a.dense ? row : i;
+    if (!in_range) {                        // an index outside the volume: nothing to read; a compact slot gets NaN
+        if (!a.dense) {
+            if (a.se_k) a.se_k[o] = NAN;
+            if (a.se_t2) a.se_t2[o] = NAN;
+            if (MODEL != T2FIT_MODEL_GAUSSIAN && a.se_sigma) a.se_sigma[o] = NAN;
+        }
+        return;
+    }
+    float y[E];
+    load_aos<E>(a.echoes, row, a.vec_ok, y);
+    double s[3];
+    se::voxel_stderr<MODEL, E>(y, a.te, a.norm != 0, __ldg(a.k + o), __ldg(a.t2 + o),
+                               MODEL == T2FIT_MODEL_GAUSSIAN ? 0.0f : __ldg(a.sigma + o), s);
+    if (a.se_k) a.se_k[o] = (float)s[0];
+    if (a.se_t2) a.se_t2[o] = (float)s[1];
+    if (MODEL != T2FIT_MODEL_GAUSSIAN && a.se_sigma) a.se_sigma[o] = (float)s[2];
+}
+
+using StderrFn = void (*)(const StderrArgs);
+
+template <int MODEL>
+StderrFn pick_stderr_e(int n_echo) {
+    switch (n_echo) {
+#define T2_CASE(E) case E: return stderr_kernel<MODEL, E>;
+        T2_CASE(2) T2_CASE(3) T2_CASE(4) T2_CASE(5) T2_CASE(6) T2_CASE(7) T2_CASE(8) T2_CASE(9) T2_CASE(10)
+        T2_CASE(11) T2_CASE(12) T2_CASE(13) T2_CASE(14) T2_CASE(15) T2_CASE(16) T2_CASE(17) T2_CASE(18)
+        T2_CASE(19) T2_CASE(20) T2_CASE(21) T2_CASE(22) T2_CASE(23) T2_CASE(24) T2_CASE(25) T2_CASE(26)
+        T2_CASE(27) T2_CASE(28) T2_CASE(29) T2_CASE(30) T2_CASE(31) T2_CASE(32)
+#undef T2_CASE
+        default: return nullptr;
+    }
+}
+
+StderrFn pick_stderr(int model, int n_echo) {
+    if (model == T2FIT_MODEL_GAUSSIAN) return pick_stderr_e<T2FIT_MODEL_GAUSSIAN>(n_echo);
+    if (model == T2FIT_MODEL_GAUSSIAN_RICIAN) return pick_stderr_e<T2FIT_MODEL_GAUSSIAN_RICIAN>(n_echo);
+    if (model == T2FIT_MODEL_RICIAN) return pick_stderr_e<T2FIT_MODEL_RICIAN>(n_echo);
+    return nullptr;
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -2223,6 +2288,41 @@ int t2fit_residuals(const t2fit_problem* p, const float* k_map, const float* t2_
     cudaStream_t st = (cudaStream_t)stream;   // NULL = the legacy default stream, as in CUDA
     residual_kernel<<<(unsigned)((p->n_fit + 255) / 256), 256, 0, st>>>(fc, p->echoes, p->mask_idx, p->n_fit, q.model, k_map,
                                                                        t2_map, sigma_map, res_map);
+    CU_TRY(cudaGetLastError());
+    return T2FIT_OK;
+}
+
+int t2fit_stderr(const t2fit_problem* p, const float* k, const float* t2, const float* sigma, int32_t dense, float* se_k,
+                 float* se_t2, float* se_sigma, void* stream) {
+    Context* c = g_ctx;
+    if (!c) return fail(T2FIT_ENOTINIT, "t2fit_init() has not succeeded");
+    if (!p) return fail(T2FIT_EINVAL, "NULL problem");
+    if (p->layout != T2FIT_LAYOUT_AOS) return fail(T2FIT_EINVAL, "t2fit_stderr reads T2FIT_LAYOUT_AOS echoes only");
+    if (p->memory != T2FIT_MEM_DEVICE) return fail(T2FIT_EINVAL, "t2fit_stderr takes T2FIT_MEM_DEVICE pointers only");
+    if (p->n_echo < 2 || p->n_echo > T2FIT_MAX_ECHO) return fail(T2FIT_EINVAL, "n_echo out of range (2..T2FIT_MAX_ECHO)");
+    if (p->model != T2FIT_MODEL_GAUSSIAN && p->model != T2FIT_MODEL_GAUSSIAN_RICIAN && p->model != T2FIT_MODEL_RICIAN)
+        return fail(T2FIT_EINVAL, "unknown model");
+    if (p->n_fit < 0 || p->n_vox < 0) return fail(T2FIT_EINVAL, "negative size");
+    if (p->idx_dtype != T2FIT_IDX_I64 && p->idx_dtype != T2FIT_IDX_I32) return fail(T2FIT_EINVAL, "bad idx_dtype");
+    if (!p->te_ms) return fail(T2FIT_EINVAL, "NULL te_ms");
+    if (p->n_fit == 0) return T2FIT_OK;
+    if (!p->echoes || !k || !t2 || (p->model != T2FIT_MODEL_GAUSSIAN && !sigma)) return fail(T2FIT_EINVAL, "NULL echoes / parameters");
+    if (!p->mask_idx && p->n_fit > p->n_vox) return fail(T2FIT_EINVAL, "n_fit > n_vox");
+    StderrArgs a{};
+    for (int e = 0; e < p->n_echo; ++e) a.te[e] = p->te_ms[e];
+    a.echoes = p->echoes;
+    if (p->mask_idx) {
+        if (p->idx_dtype == T2FIT_IDX_I32) a.idx32 = reinterpret_cast<const int32_t*>(p->mask_idx);
+        else a.idx = p->mask_idx;
+    }
+    a.n_fit = p->n_fit; a.n_vox = p->n_vox;
+    a.k = k; a.t2 = t2; a.sigma = sigma;
+    a.se_k = se_k; a.se_t2 = se_t2; a.se_sigma = se_sigma;
+    a.dense = dense != 0; a.norm = p->norm != 0;
+    a.vec_ok = (reinterpret_cast<uintptr_t>(p->echoes) % 16) == 0;
+    const StderrFn fn = pick_stderr(p->model, p->n_echo);
+    CU_TRY(cudaSetDevice(c->device));
+    fn<<<(unsigned)((p->n_fit + 255) / 256), 256, 0, (cudaStream_t)stream>>>(a);
     CU_TRY(cudaGetLastError());
     return T2FIT_OK;
 }

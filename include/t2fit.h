@@ -26,7 +26,7 @@
 extern "C" {
 #endif
 
-#define T2FIT_ABI_VERSION 4
+#define T2FIT_ABI_VERSION 5
 #define T2FIT_MAX_ECHO 32
 #define T2FIT_MAX_DUP 7 /* peer destinations of the fused all-gather: the other GPUs of an 8-GPU node */
 
@@ -262,6 +262,26 @@ int t2fit_scatter(const float *const *compact, float *const *dense, int32_t n_ma
  * maps are dense [n_vox] device arrays.  t2fit_run already returns the same residuals. */
 int t2fit_residuals(const t2fit_problem *p, const float *k_map, const float *t2_map, const float *sigma_map,
                     float *res_map, void *stream);
+
+/* Per-voxel standard errors of the fitted parameters (DESIGN.md section 11), at the parameters given: the unconstrained local
+ * linearisation of the fit's objective, bounds ignored, FP64 per voxel (csrc/t2fit_stderr.cuh).
+ *   gaussian, gaussian_rician: Cov = s^2 (J'J)^-1, J[e][j] = d model_e / d theta_j, s^2 = sum_e r_e^2 / (E - P)
+ *                              (scipy.optimize.curve_fit's pcov with absolute_sigma=False)
+ *   rician:                    Cov = H^-1, H the analytic Hessian of the summed negative log-likelihood (rician_obj :157-177)
+ * theta = (k, T2[, sigma]) in the units of the maps; se_j = sqrt(Cov_jj) from a Cholesky factorisation of D A D,
+ * D = diag(A_jj^-1/2).  The echoes are those of the fit: float32, scaled by y / max(y) in float32 when p->norm.
+ * NaN rule: all standard errors of a voxel are NaN when an echo is not finite (rician: or <= 0), a parameter is not finite
+ * or T2 <= 0, n_echo <= P, a diagonal entry of A is <= 0, or a Cholesky pivot is <= 0 or not finite; otherwise they are
+ * finite (huge for a near-singular voxel: reported, not clipped).
+ * Reads echoes / layout / memory / mask_idx / idx_dtype / n_vox / n_fit / n_echo / te_ms / model / norm of *p, as
+ * t2fit_residuals; T2FIT_LAYOUT_AOS and T2FIT_MEM_DEVICE only.  k, t2 (and sigma for the 3-parameter models) are device
+ * float32 parameters: dense == 0 compact [n_fit] (element i = voxel mask_idx[i]), dense != 0 [n_vox] maps indexed by row.
+ * se_k / se_t2 / se_sigma are written the same way; any may be NULL (skipped); se_sigma is not written for gaussian.  A
+ * mask_idx entry outside [0, n_vox) reads nothing and gives NaN in a compact output (a dense one is left untouched).
+ * Asynchronous on `stream`.  EINVAL: bad layout / memory kind, NULL pointers, n_echo outside 2..T2FIT_MAX_ECHO;
+ * ENOTINIT before t2fit_init.  n_fit == 0 is a no-op. */
+int t2fit_stderr(const t2fit_problem *p, const float *k, const float *t2, const float *sigma, int32_t dense, float *se_k,
+                 float *se_t2, float *se_sigma, void *stream);
 
 /* Algorithmic work of the shipped kernels, for roofline accounting (DESIGN.md): FLOPs and MUFU ops
  * of one pass over the echoes, and the fixed per-voxel part. */
