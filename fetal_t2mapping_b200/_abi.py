@@ -126,6 +126,8 @@ SYMBOLS = [
     ("t2fit_residuals", C.c_int, [C.POINTER(Problem), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     ("t2fit_stderr", C.c_int, [C.POINTER(Problem), C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p,
                                C.c_void_p, C.c_void_p]),
+    ("t2fit_t2_interval", C.c_int, [C.POINTER(Problem), C.c_double, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p,
+                                    C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     ("t2fit_work_model", C.c_int, [C.c_int32, C.c_int32] + [C.POINTER(C.c_double)] * 5),
 ]
 

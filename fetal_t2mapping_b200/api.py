@@ -25,7 +25,7 @@ import numpy as np
 from . import _abi
 from .presets import NO_PRIOR_K_UB, NO_PRIOR_T2_BOUNDS
 
-__all__ = ["fit_voxels_batch", "fit_voxels_into", "check_counts", "t2map_volume", "compute_residuals", "parameter_stderr", "FitResult", "init",
+__all__ = ["fit_voxels_batch", "fit_voxels_into", "check_counts", "t2map_volume", "compute_residuals", "parameter_stderr", "t2_interval", "FitResult", "init",
            "shutdown", "device_info", "mask_indices_device", "work_model", "pinned_array", "BOUNDS_ERROR"]
 
 BOUNDS_ERROR = "An upper bound is less than the corresponding lower bound."   # scipy's text
@@ -327,6 +327,52 @@ def _stderr_staged(lib, p, fit, rows, k, t2, sigma):
     return o[0], o[1], (o[2] if fit != "gaussian" else None)
 
 
+def _interval_q(fit, n_echo, level):
+    """The quantile q of t2fit_t2_interval for a confidence level: t^2_{E-P}(1 - alpha/2) for the least-squares fits (the
+    profile-t interval), chi^2_1(level) for 'rician' (the likelihood ratio).  E <= P leaves no residual degrees of freedom:
+    every voxel is invalid then, and q is only a placeholder."""
+    from scipy import stats
+    if not 0.0 < float(level) < 1.0:
+        raise ValueError("level must lie in (0, 1)")
+    if fit == "rician":
+        return float(stats.chi2.ppf(level, 1))
+    dof = n_echo - (2 if fit == "gaussian" else 3)
+    return float(stats.t.ppf(0.5 + 0.5 * level, dof) ** 2) if dof > 0 else 0.0
+
+
+def interval_grid(t2_lo, t2_hi, n_grid=64):
+    """The T2 grid of the interval pass: ``T2_g = t2_lo (t2_hi / t2_lo)^(g / (n_grid - 1))``, both bounds included."""
+    t = t2_lo * np.power(t2_hi / t2_lo, np.arange(n_grid, dtype=np.float64) / (n_grid - 1))
+    t[-1] = t2_hi
+    return t
+
+
+def _interval_launch(lib, p, q, n_grid, dense, outs, profile, stream):
+    """t2fit_t2_interval on the echoes / indices / sizes already in ``p`` (device AoS): ``outs`` (lo, hi, best, flags) and
+    ``profile`` are device addresses or None."""
+    _abi.check(lib, lib.t2fit_t2_interval(C.byref(p), q, int(n_grid), int(dense), *outs, profile, stream), "t2fit_t2_interval")
+
+
+def _interval_staged(lib, p, rows, q, n_grid, profile):
+    """The interval of host rows ``rows`` [M, E]: staged to the device through torch, results copied back as numpy
+    (lo, hi, best float32 [M], flags uint8 [M], profile float64 [M, n_grid] or None)."""
+    import torch
+    dev = torch.device("cuda", _state["device"])
+    m = rows.shape[0]
+    y = torch.from_numpy(np.ascontiguousarray(rows, dtype=np.float32)).to(dev)
+    f = torch.empty((3, m), dtype=torch.float32, device=dev)
+    fl = torch.empty(m, dtype=torch.uint8, device=dev)
+    pr = torch.empty((m, n_grid), dtype=torch.float64, device=dev) if profile else None
+    q_ = _abi.Problem.from_buffer_copy(p)
+    q_.echoes, q_.memory, q_.layout, q_.mask_idx, q_.idx_dtype = y.data_ptr(), _abi.MEM_DEVICE, _abi.LAYOUT_AOS, None, _abi.IDX_I64
+    q_.n_vox, q_.n_fit, q_.ld = m, m, 0
+    if m:
+        _interval_launch(lib, q_, q, n_grid, 0, [f[0].data_ptr(), f[1].data_ptr(), f[2].data_ptr(), fl.data_ptr()],
+                         pr.data_ptr() if pr is not None else None, torch.cuda.current_stream(dev).cuda_stream)
+    o = f.cpu().numpy()
+    return o[0], o[1], o[2], fl.cpu().numpy(), (pr.cpu().numpy() if pr is not None else None)
+
+
 def fit_voxels_batch(reshaped_t2w, mask_indices, TEeffs, fit, fit_params, prior=True, norm=False, *,
                      solver="auto", trace_cap=0, max_iter=0, tol=0.0, init_mode="auto", check_bounds=True,
                      dense_out=None, want=("nit", "fun", "status")) -> FitResult:
@@ -512,12 +558,15 @@ def mask_indices_device(mask, n_masks=None):
     return idx[:n.value]
 
 
-def t2map_volume(t2w, mask, TEeffs, fit, fit_params, prior=True, norm=False, stderr=False, **kw):
+def t2map_volume(t2w, mask, TEeffs, fit, fit_params, prior=True, norm=False, stderr=False, t2_interval=None, **kw):
     """Stacked per-TE volumes ``t2w[z,y,x,E]``, mask ``[z,y,x]`` or per-TE masks ``[z,y,x,E]`` and the
     TE vector in; ``(t2_map, k_map, sigma_map, res_map)`` float32 ``[z,y,x]`` out, zeros off-mask --
     the whole hot block of ``process_t2maps`` (run_t2mapping.py:383-386, :411-461, :471-473).
     ``stderr=True`` adds a fifth element ``(se_t2_map, se_k_map, se_sigma_map)``: the standard errors of the fitted
-    parameters (:func:`parameter_stderr`), float32 ``[z,y,x]``, zeros off-mask (se_sigma all zeros for 'gaussian')."""
+    parameters (:func:`parameter_stderr`), float32 ``[z,y,x]``, zeros off-mask (se_sigma all zeros for 'gaussian').
+    ``t2_interval=level`` (e.g. 0.95) appends ``(t2_lo_map, t2_hi_map, t2_best_map, flags_map)`` as the last element: the
+    profile-likelihood confidence interval for T2 at that level (:func:`t2_interval`, default grid), float32 / uint8
+    ``[z,y,x]``, zeros off-mask."""
     lib = init()
     shape3 = tuple(t2w.shape[:3])
     n_echo = t2w.shape[-1]
@@ -571,19 +620,34 @@ def t2map_volume(t2w, mask, TEeffs, fit, fit_params, prior=True, norm=False, std
     elif o.status_count[3] > 0:
         raise ValueError(BOUNDS_ERROR)
     out = tuple(maps[i].reshape(shape3) for i in range(4))
-    if not stderr:
+    if not stderr and t2_interval is None:
         return out
-    if stream is not None:
-        se = torch.zeros((3, n_vox), dtype=torch.float32, device=y.device)
-        if m:
-            _stderr_launch(lib, p, fit, [mp[1], mp[0], mp[2]], 1, [se[1].data_ptr(), se[0].data_ptr(), se[2].data_ptr()], stream)
-    else:
-        se = np.zeros((3, n_vox), np.float32)
-        sk, st, ss = _stderr_staged(lib, p, fit, y[idx], maps[1][idx], maps[0][idx], maps[2][idx])
-        se[0][idx], se[1][idx] = st, sk
-        if ss is not None:
-            se[2][idx] = ss
-    return out + (tuple(se[i].reshape(shape3) for i in range(3)),)
+    if stderr:
+        if stream is not None:
+            se = torch.zeros((3, n_vox), dtype=torch.float32, device=y.device)
+            if m:
+                _stderr_launch(lib, p, fit, [mp[1], mp[0], mp[2]], 1, [se[1].data_ptr(), se[0].data_ptr(), se[2].data_ptr()], stream)
+        else:
+            se = np.zeros((3, n_vox), np.float32)
+            sk, st, ss = _stderr_staged(lib, p, fit, y[idx], maps[1][idx], maps[0][idx], maps[2][idx])
+            se[0][idx], se[1][idx] = st, sk
+            if ss is not None:
+                se[2][idx] = ss
+        out = out + (tuple(se[i].reshape(shape3) for i in range(3)),)
+    if t2_interval is not None:
+        q, G = _interval_q(fit, n_echo, t2_interval), 64
+        if stream is not None:
+            iv = torch.zeros((3, n_vox), dtype=torch.float32, device=y.device)
+            ivf = torch.zeros(n_vox, dtype=torch.uint8, device=y.device)
+            if m:
+                _interval_launch(lib, p, q, G, 1, [iv[0].data_ptr(), iv[1].data_ptr(), iv[2].data_ptr(), ivf.data_ptr()], None,
+                                 stream)
+        else:
+            iv = np.zeros((3, n_vox), np.float32)
+            ivf = np.zeros(n_vox, np.uint8)
+            iv[0][idx], iv[1][idx], iv[2][idx], ivf[idx], _ = _interval_staged(lib, p, y[idx], q, G, False)
+        out = out + (tuple(iv[i].reshape(shape3) for i in range(3)) + (ivf.reshape(shape3),),)
+    return out
 
 
 def compute_residuals(reshaped_t2w, TEeffs, fit, norm, k_map, t2_map, sigma_map, res_map, mask_indices, mask):
@@ -656,3 +720,67 @@ def parameter_stderr(reshaped_t2w, TEeffs, fit, norm, k_map, t2_map, sigma_map, 
     if host:
         se = se.cpu().numpy()
     return tuple(se[i].reshape(shape3) for i in range(3))
+
+
+def t2_interval(reshaped_t2w, mask_indices, TEeffs, fit, fit_params, prior=True, norm=False, *, level=0.95, n_grid=64,
+                profile=False):
+    """Profile-likelihood confidence interval for T2 of every voxel ``mask_indices[i]`` of ``reshaped_t2w`` (float32
+    ``[N, E]``; ``mask_indices`` None = all rows), with the arguments of :func:`fit_voxels_batch`.  Runs the CUDA pass
+    ``t2fit_t2_interval`` (FP64 per voxel).  Returns compact ``(t2_lo, t2_hi, t2_best, flags)`` -- float32, float32,
+    float32, uint8 ``[M]`` -- and with ``profile=True`` also ``profile`` float64 ``[M, n_grid]`` (p at the grid) and
+    ``grid`` float64 ``[n_grid]`` (the T2 values).  numpy input gives numpy output (the masked rows are staged through
+    torch); a CUDA tensor gives CUDA tensors, asynchronously on the current stream.
+
+    Definition (DESIGN.md section 12): with the fit's objective f (mean squared error for 'gaussian' / 'gaussian_rician',
+    summed negative log-likelihood for 'rician') and the fit's box, ``p(T2) = min over (k[, sigma]) of f``; the interval
+    is the hull of ``{T2 : p(T2) <= thr}``, ``thr = p* (1 + q / (E - P))`` with ``q = t^2_{E-P}((1 + level) / 2)`` for the
+    least-squares fits, ``thr = p* + q / 2`` with ``q = chi^2_1(level)`` for 'rician'; ``t2_best`` is the T2 of the
+    bounded minimiser.  ``flags``: 1 t2_lo is the lower T2 bound, 2 t2_hi is the upper T2 bound (upper end not
+    determined), 4 the set is not one interval at grid resolution, 8 invalid (NaN; non-finite echoes, rician echoes <= 0,
+    E <= P, the --no_prior voxel with S(TE0) above the k bound).  The interval does not depend on the fit's point, so it is
+    the same whichever solver fits the maps.  ``n_grid``: 16..256 grid points (default 64)."""
+    import torch
+    lib = init()
+    p = _abi.Problem()
+    keep = [_fill_problem(p, fit, fit_params, TEeffs, prior, norm, 0, 0.0, "auto")]
+    q = _interval_q(fit, p.n_echo, level)
+    if not 16 <= int(n_grid) <= 256:
+        raise ValueError("n_grid must lie in 16..256")
+    t_lo, t_hi = (NO_PRIOR_T2_BOUNDS if not prior else (p.lb[1], p.ub[1]))
+    if _is_torch(reshaped_t2w):
+        y = reshaped_t2w
+        if not y.is_cuda or y.dtype != torch.float32 or not y.is_contiguous() or y.dim() != 2:
+            raise ValueError("device input must be a contiguous float32 CUDA tensor [N, E]")
+        if y.device.index != _state["device"]:
+            raise ValueError(f"tensor on cuda:{y.device.index}, library bound to cuda:{_state['device']}")
+        if y.shape[1] != p.n_echo:
+            raise ValueError(f"reshaped_t2w has {y.shape[1]} echoes, TEeffs has {p.n_echo}")
+        idx = mask_indices
+        if idx is not None:
+            if not _is_torch(idx):
+                idx = np.asarray(idx)
+                idx = torch.as_tensor(np.ascontiguousarray(idx, dtype=np.int32 if idx.dtype == np.int32 else np.int64), device=y.device)
+            if idx.dtype not in (torch.int64, torch.int32) or not idx.is_contiguous():
+                idx = idx.to(torch.int64).contiguous()
+            p.idx_dtype = _abi.IDX_I32 if idx.dtype == torch.int32 else _abi.IDX_I64
+        m = y.shape[0] if idx is None else idx.numel()
+        f = torch.empty((3, m), dtype=torch.float32, device=y.device)
+        fl = torch.empty(m, dtype=torch.uint8, device=y.device)
+        pr = torch.empty((m, n_grid), dtype=torch.float64, device=y.device) if profile else None
+        p.echoes, p.memory, p.layout, p.ld = y.data_ptr(), _abi.MEM_DEVICE, _abi.LAYOUT_AOS, 0
+        p.mask_idx = idx.data_ptr() if idx is not None else None
+        p.n_vox, p.n_fit = y.shape[0], m
+        _interval_launch(lib, p, q, n_grid, 0, [f[0].data_ptr(), f[1].data_ptr(), f[2].data_ptr(), fl.data_ptr()],
+                         pr.data_ptr() if pr is not None else None, torch.cuda.current_stream(y.device).cuda_stream)
+        keep += [y, idx]
+        lo, hi, best = f[0], f[1], f[2]
+    else:
+        y = np.asarray(reshaped_t2w)
+        if y.ndim != 2 or y.shape[1] != p.n_echo:
+            raise ValueError(f"reshaped_t2w must be [N, {p.n_echo}]")
+        rows = y if mask_indices is None else y[np.asarray(mask_indices)]
+        lo, hi, best, fl, pr = _interval_staged(lib, p, rows, q, n_grid, profile)
+    del keep
+    if not profile:
+        return lo, hi, best, fl
+    return lo, hi, best, fl, pr, interval_grid(t_lo, t_hi, n_grid)

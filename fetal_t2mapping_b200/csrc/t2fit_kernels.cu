@@ -41,6 +41,7 @@
 #include "t2fit_lbfgsb_coop.cuh"
 #include "t2fit_lbfgsb_dense.cuh"
 #include "t2fit_stderr.cuh"
+#include "t2fit_interval.cuh"
 #include "t2fit_workers.h"
 
 using namespace t2fit;
@@ -1077,6 +1078,77 @@ StderrFn pick_stderr(int model, int n_echo) {
     if (model == T2FIT_MODEL_GAUSSIAN_RICIAN) return pick_stderr_e<T2FIT_MODEL_GAUSSIAN_RICIAN>(n_echo);
     if (model == T2FIT_MODEL_RICIAN) return pick_stderr_e<T2FIT_MODEL_RICIAN>(n_echo);
     return nullptr;
+}
+
+// ------------------------------------------------------------------------------------------------
+// interval_kernel: per-voxel profile-likelihood interval for T2 (t2fit_t2_interval, csrc/t2fit_interval.cuh).
+// One thread per voxel, FP64.  The kernel is instantiated per echo count for the row load only; the model is a run-time
+// argument and the profile work is one out-of-line routine with E at run time, so its code is compiled 31 times rather than
+// 93 (ptxas gives every kernel its own copy of the routine).  The grid work space (iv::Grid, 6 KB) is thread-local memory.
+// ------------------------------------------------------------------------------------------------
+struct IntervalArgs {
+    double te[kMaxEcho];
+    iv::Box box;               // k / T2 / sigma bounds in force; k_lo replaced by y(TE_0) per voxel when no_prior
+    double q;
+    const float* echoes;
+    const int64_t* idx;        // at most one of idx / idx32 is set; neither = rows 0..n_fit-1
+    const int32_t* idx32;
+    int64_t n_fit, n_vox;
+    float *lo, *hi, *best;
+    uint8_t* flags;
+    double* profile;           // [n_fit, n_grid] or NULL
+    int model;
+    int n_grid;
+    int dense;                 // lo / hi / best / flags indexed by row instead of i
+    int norm;
+    int no_prior;
+    int vec_ok;
+};
+
+template <int E>
+__global__ void __launch_bounds__(128) interval_kernel(const __grid_constant__ IntervalArgs a) {
+    const int64_t i = (int64_t)blockIdx.x * 128 + threadIdx.x;
+    if (i >= a.n_fit) return;
+    const int64_t row = a.idx ? __ldg(a.idx + i) : a.idx32 ? (int64_t)__ldg(a.idx32 + i) : i;
+    const bool in_range = (unsigned long long)row < (unsigned long long)a.n_vox;
+    const int64_t o = a.dense ? row : i;
+    double* prof = a.profile ? a.profile + i * a.n_grid : nullptr;
+    if (!in_range) {                        // an index outside the volume: nothing to read; a compact slot gets NaN / invalid
+        if (!a.dense) {
+            if (a.lo) a.lo[o] = NAN;
+            if (a.hi) a.hi[o] = NAN;
+            if (a.best) a.best[o] = NAN;
+            if (a.flags) a.flags[o] = iv::kInvalid;
+        }
+        if (prof) for (int g = 0; g < a.n_grid; ++g) prof[g] = NAN;
+        return;
+    }
+    float y[E];
+    load_aos<E>(a.echoes, row, a.vec_ok, y);
+    iv::Voxel v;
+    iv::Grid w;
+    const bool ok = iv::load_voxel<E>(y, a.te, a.model, a.norm != 0, a.box, a.no_prior != 0, v);
+    double lo, hi, best;
+    int fl;
+    iv::voxel_interval(v, ok, a.q, a.n_grid, w, lo, hi, best, fl, prof);
+    if (a.lo) a.lo[o] = (float)lo;
+    if (a.hi) a.hi[o] = (float)hi;
+    if (a.best) a.best[o] = (float)best;
+    if (a.flags) a.flags[o] = (uint8_t)fl;
+}
+
+using IntervalFn = void (*)(const IntervalArgs);
+
+IntervalFn pick_interval(int n_echo) {
+    switch (n_echo) {
+#define T2_CASE(E) case E: return interval_kernel<E>;
+        T2_CASE(2) T2_CASE(3) T2_CASE(4) T2_CASE(5) T2_CASE(6) T2_CASE(7) T2_CASE(8) T2_CASE(9) T2_CASE(10)
+        T2_CASE(11) T2_CASE(12) T2_CASE(13) T2_CASE(14) T2_CASE(15) T2_CASE(16) T2_CASE(17) T2_CASE(18)
+        T2_CASE(19) T2_CASE(20) T2_CASE(21) T2_CASE(22) T2_CASE(23) T2_CASE(24) T2_CASE(25) T2_CASE(26)
+        T2_CASE(27) T2_CASE(28) T2_CASE(29) T2_CASE(30) T2_CASE(31) T2_CASE(32)
+#undef T2_CASE
+        default: return nullptr;
+    }
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -2323,6 +2395,50 @@ int t2fit_stderr(const t2fit_problem* p, const float* k, const float* t2, const 
     const StderrFn fn = pick_stderr(p->model, p->n_echo);
     CU_TRY(cudaSetDevice(c->device));
     fn<<<(unsigned)((p->n_fit + 255) / 256), 256, 0, (cudaStream_t)stream>>>(a);
+    CU_TRY(cudaGetLastError());
+    return T2FIT_OK;
+}
+
+int t2fit_t2_interval(const t2fit_problem* p, double q, int32_t n_grid, int32_t dense, float* t2_lo, float* t2_hi,
+                      float* t2_best, uint8_t* flags, double* profile, void* stream) {
+    Context* c = g_ctx;
+    if (!c) return fail(T2FIT_ENOTINIT, "t2fit_init() has not succeeded");
+    if (!p) return fail(T2FIT_EINVAL, "NULL problem");
+    if (p->layout != T2FIT_LAYOUT_AOS) return fail(T2FIT_EINVAL, "t2fit_t2_interval reads T2FIT_LAYOUT_AOS echoes only");
+    if (p->memory != T2FIT_MEM_DEVICE) return fail(T2FIT_EINVAL, "t2fit_t2_interval takes T2FIT_MEM_DEVICE pointers only");
+    if (p->n_echo < 2 || p->n_echo > T2FIT_MAX_ECHO) return fail(T2FIT_EINVAL, "n_echo out of range (2..T2FIT_MAX_ECHO)");
+    if (p->model != T2FIT_MODEL_GAUSSIAN && p->model != T2FIT_MODEL_GAUSSIAN_RICIAN && p->model != T2FIT_MODEL_RICIAN)
+        return fail(T2FIT_EINVAL, "unknown model");
+    if (p->n_fit < 0 || p->n_vox < 0) return fail(T2FIT_EINVAL, "negative size");
+    if (p->idx_dtype != T2FIT_IDX_I64 && p->idx_dtype != T2FIT_IDX_I32) return fail(T2FIT_EINVAL, "bad idx_dtype");
+    if (!p->te_ms) return fail(T2FIT_EINVAL, "NULL te_ms");
+    if (n_grid < iv::kMinGrid || n_grid > iv::kMaxGrid) return fail(T2FIT_EINVAL, "n_grid out of range (16..256)");
+    if (!(q >= 0.0) || !(q - q == 0.0)) return fail(T2FIT_EINVAL, "q must be finite and >= 0");
+    iv::Box b{p->lb[0], p->ub[0], p->lb[1], p->ub[1], p->lb[2], p->ub[2]};
+    if (p->no_prior) { b.k_hi = p->no_prior_k_ub; b.t_lo = p->no_prior_t2_lb; b.t_hi = p->no_prior_t2_ub; }
+    if (!(b.t_lo > 0.0) || !(b.t_lo < b.t_hi) || !(b.t_hi - b.t_hi == 0.0))
+        return fail(T2FIT_EINVAL, "the T2 bounds must be finite with 0 < lb < ub");
+    if (p->model == T2FIT_MODEL_GAUSSIAN) b.s_lo = b.s_hi = 1.0;
+    else if (!(b.s_lo > 0.0)) return fail(T2FIT_EINVAL, "the sigma lower bound must be > 0");
+    if (p->n_fit == 0) return T2FIT_OK;
+    if (!p->echoes) return fail(T2FIT_EINVAL, "NULL echoes");
+    if (!p->mask_idx && p->n_fit > p->n_vox) return fail(T2FIT_EINVAL, "n_fit > n_vox");
+    IntervalArgs a{};
+    for (int e = 0; e < p->n_echo; ++e) a.te[e] = p->te_ms[e];
+    a.box = b;
+    a.q = q;
+    a.echoes = p->echoes;
+    if (p->mask_idx) {
+        if (p->idx_dtype == T2FIT_IDX_I32) a.idx32 = reinterpret_cast<const int32_t*>(p->mask_idx);
+        else a.idx = p->mask_idx;
+    }
+    a.n_fit = p->n_fit; a.n_vox = p->n_vox;
+    a.lo = t2_lo; a.hi = t2_hi; a.best = t2_best; a.flags = flags; a.profile = profile;
+    a.model = p->model; a.n_grid = n_grid; a.dense = dense != 0; a.norm = p->norm != 0; a.no_prior = p->no_prior != 0;
+    a.vec_ok = (reinterpret_cast<uintptr_t>(p->echoes) % 16) == 0;
+    const IntervalFn fn = pick_interval(p->n_echo);
+    CU_TRY(cudaSetDevice(c->device));
+    fn<<<(unsigned)((p->n_fit + 127) / 128), 128, 0, (cudaStream_t)stream>>>(a);
     CU_TRY(cudaGetLastError());
     return T2FIT_OK;
 }

@@ -283,6 +283,32 @@ int t2fit_residuals(const t2fit_problem *p, const float *k_map, const float *t2_
 int t2fit_stderr(const t2fit_problem *p, const float *k, const float *t2, const float *sigma, int32_t dense, float *se_k,
                  float *se_t2, float *se_sigma, void *stream);
 
+/* Per-voxel profile-likelihood confidence interval for T2 (DESIGN.md section 12), FP64 per voxel (csrc/t2fit_interval.cuh).
+ * For one voxel, with the fit's objective f (gaussian, gaussian_rician: the mean squared error; rician: the summed negative
+ * log-likelihood of rician_obj :157-177) on the fit's echoes (float32, scaled by y / max(y) in float32 when p->norm) and
+ * the fit's box (lb / ub, or under p->no_prior k in [y(TE_0), no_prior_k_ub] and T2 in [no_prior_t2_lb, no_prior_t2_ub],
+ * sigma keeping lb[2] / ub[2]):
+ *   p(T2) = min over (k[, sigma]) in the box of f;  p* = min over T2 in the box of p, reached at t2_best;
+ *   the set {T2 : p(T2) <= thr}, thr = p* (1 + q / (E - P)) for the least-squares fits (q = t^2_{E-P}(1 - alpha/2), the
+ *   profile-t interval), thr = p* + q / 2 for rician (q = chi^2_1(1 - alpha), the likelihood ratio);
+ *   t2_lo / t2_hi = the smallest / largest member of the set (its hull when it is not connected).
+ * flags: bit 0 t2_lo is the lower T2 bound; bit 1 t2_hi is the upper T2 bound (upper end not determined); bit 2 a grid
+ * point strictly between t2_lo and t2_hi lies outside the set; bit 3 invalid: t2_lo / t2_hi / t2_best NaN, when an echo is
+ * not finite (rician: or <= 0), n_echo <= P, the box is empty (--no_prior with y(TE_0) > no_prior_k_ub: the fit's status
+ * 3) or p* is not finite.  A least-squares voxel with p* == 0 is valid; its set is where p == 0.
+ * Procedure: p on n_grid (16..256) points T2_g = lb (ub/lb)^(g/(n_grid-1)); golden-section refinement of p* / t2_best
+ * (relative T2 tolerance 1e-7 or better); bisection of the crossings that bound the hull (1e-6 or better).
+ * Reads echoes / layout / memory / mask_idx / idx_dtype / n_vox / n_fit / n_echo / te_ms / model / norm / lb / ub / no_prior*
+ * of *p; T2FIT_LAYOUT_AOS and T2FIT_MEM_DEVICE only.  dense == 0: t2_lo / t2_hi / t2_best / flags compact [n_fit] (element
+ * i = voxel mask_idx[i]); dense != 0: [n_vox] indexed by row.  profile (optional): [n_fit, n_grid] float64 p(T2_g), compact
+ * in either case (NaN for an invalid voxel).  Any output may be NULL (skipped).  A mask_idx entry outside [0, n_vox) reads
+ * nothing: NaN and flag 8 in a compact output (a dense one is left untouched).  Asynchronous on `stream`.
+ * EINVAL: bad layout / memory kind, NULL echoes / te_ms, n_echo outside 2..T2FIT_MAX_ECHO, n_grid outside 16..256, q not
+ * finite or < 0, T2 bounds not finite with 0 < lb < ub, a sigma lower bound <= 0 (3-parameter models); ENOTINIT before
+ * t2fit_init.  n_fit == 0 is a no-op. */
+int t2fit_t2_interval(const t2fit_problem *p, double q, int32_t n_grid, int32_t dense, float *t2_lo, float *t2_hi,
+                      float *t2_best, uint8_t *flags, double *profile, void *stream);
+
 /* Algorithmic work of the shipped kernels, for roofline accounting (DESIGN.md): FLOPs and MUFU ops
  * of one pass over the echoes, and the fixed per-voxel part. */
 int t2fit_work_model(int32_t model, int32_t n_echo, double *flop_per_pass, double *mufu_per_pass,
