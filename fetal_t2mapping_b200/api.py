@@ -308,23 +308,29 @@ def _stderr_launch(lib, p, fit, params, dense, se, stream):
                "t2fit_stderr")
 
 
-def _stderr_staged(lib, p, fit, rows, k, t2, sigma):
-    """Standard errors of host rows ``rows`` [M, E] at compact host parameters: rows and parameters are staged to the
-    device through torch (as :func:`compute_residuals` does), the results copied back as float32 numpy [M] arrays."""
+def _stderr_pass(lib, p, fit, k, t2, sigma, dense):
+    """t2fit_stderr on the device rows of ``p`` at the float32 device parameters ``k``, ``t2``, ``sigma`` (None for
+    'gaussian'), on the current stream of their GPU.  Returns float32 [3, n] (se_k, se_t2, se_sigma): n = p.n_vox, zeros
+    off the index, when ``dense``, else n = p.n_fit with se_sigma unset for 'gaussian'."""
+    import torch
+    se = (torch.zeros if dense else torch.empty)((3, p.n_vox if dense else p.n_fit), dtype=torch.float32, device=k.device)
+    _stderr_launch(lib, p, fit, [k.data_ptr(), t2.data_ptr(), sigma.data_ptr() if sigma is not None else None], dense,
+                   [se[i].data_ptr() for i in range(3)], torch.cuda.current_stream(k.device).cuda_stream)
+    return se
+
+
+def _staged(p, rows, *params):
+    """Host input for a device pass: a copy of ``p`` that reads ``rows`` [M, E], copied to the bound GPU, without an
+    index (rows 0..M-1, so dense and compact output slots coincide), and the device tensors [rows, *params], each per-row
+    array of ``params`` copied as float32 (None stays None).  The tensors must stay alive for the pass."""
     import torch
     dev = torch.device("cuda", _state["device"])
-    m = rows.shape[0]
     y = torch.from_numpy(np.ascontiguousarray(rows, dtype=np.float32)).to(dev)
-    par = [torch.from_numpy(np.ascontiguousarray(a, dtype=np.float32)).to(dev) if a is not None else None for a in (k, t2, sigma)]
-    out = torch.zeros((3, m), dtype=torch.float32, device=dev)
     q = _abi.Problem.from_buffer_copy(p)
     q.echoes, q.memory, q.layout, q.mask_idx, q.idx_dtype = y.data_ptr(), _abi.MEM_DEVICE, _abi.LAYOUT_AOS, None, _abi.IDX_I64
-    q.n_vox, q.n_fit, q.ld = m, m, 0
-    if m:
-        _stderr_launch(lib, q, fit, [t.data_ptr() if t is not None else None for t in par], 0,
-                       [out[i].data_ptr() for i in range(3)], torch.cuda.current_stream(dev).cuda_stream)
-    o = out.cpu().numpy()
-    return o[0], o[1], (o[2] if fit != "gaussian" else None)
+    q.n_vox, q.n_fit, q.ld = y.shape[0], y.shape[0], 0
+    return q, [y] + [torch.from_numpy(np.ascontiguousarray(a, dtype=np.float32)).to(dev) if a is not None else None
+                     for a in params]
 
 
 def _interval_q(fit, n_echo, level):
@@ -353,24 +359,44 @@ def _interval_launch(lib, p, q, n_grid, dense, outs, profile, stream):
     _abi.check(lib, lib.t2fit_t2_interval(C.byref(p), q, int(n_grid), int(dense), *outs, profile, stream), "t2fit_t2_interval")
 
 
-def _interval_staged(lib, p, rows, q, n_grid, profile):
-    """The interval of host rows ``rows`` [M, E]: staged to the device through torch, results copied back as numpy
-    (lo, hi, best float32 [M], flags uint8 [M], profile float64 [M, n_grid] or None)."""
+def _interval_pass(lib, p, q, n_grid, dense, profile, device):
+    """t2fit_t2_interval on the device rows of ``p`` on the current stream of ``device``.  Returns (f, flags, prof): f
+    float32 [3, n] (lo, hi, best), flags uint8 [n] -- n = p.n_vox, zeros off the index, when ``dense``, else p.n_fit --
+    and with ``profile`` p at the grid, float64 [p.n_fit, n_grid], else None."""
     import torch
-    dev = torch.device("cuda", _state["device"])
-    m = rows.shape[0]
-    y = torch.from_numpy(np.ascontiguousarray(rows, dtype=np.float32)).to(dev)
-    f = torch.empty((3, m), dtype=torch.float32, device=dev)
-    fl = torch.empty(m, dtype=torch.uint8, device=dev)
-    pr = torch.empty((m, n_grid), dtype=torch.float64, device=dev) if profile else None
-    q_ = _abi.Problem.from_buffer_copy(p)
-    q_.echoes, q_.memory, q_.layout, q_.mask_idx, q_.idx_dtype = y.data_ptr(), _abi.MEM_DEVICE, _abi.LAYOUT_AOS, None, _abi.IDX_I64
-    q_.n_vox, q_.n_fit, q_.ld = m, m, 0
-    if m:
-        _interval_launch(lib, q_, q, n_grid, 0, [f[0].data_ptr(), f[1].data_ptr(), f[2].data_ptr(), fl.data_ptr()],
-                         pr.data_ptr() if pr is not None else None, torch.cuda.current_stream(dev).cuda_stream)
-    o = f.cpu().numpy()
-    return o[0], o[1], o[2], fl.cpu().numpy(), (pr.cpu().numpy() if pr is not None else None)
+    new, n = (torch.zeros, p.n_vox) if dense else (torch.empty, p.n_fit)
+    f = new((3, n), dtype=torch.float32, device=device)
+    fl = new(n, dtype=torch.uint8, device=device)
+    pr = torch.empty((p.n_fit, n_grid), dtype=torch.float64, device=device) if profile else None
+    _interval_launch(lib, p, q, n_grid, dense, [f[0].data_ptr(), f[1].data_ptr(), f[2].data_ptr(), fl.data_ptr()],
+                     pr.data_ptr() if pr is not None else None, torch.cuda.current_stream(device).cuda_stream)
+    return f, fl, pr
+
+
+def _device_rows(p, reshaped_t2w, mask_indices):
+    """Points ``p`` at device echo rows: ``reshaped_t2w`` must be a contiguous float32 CUDA tensor [N, p.n_echo] on the
+    bound GPU.  ``mask_indices`` (numpy or torch on any device; None = every row) is brought to that GPU, int32 kept as
+    int32 (half the index bytes), anything else as contiguous int64.  Returns the index tensor, which must stay alive for
+    the call."""
+    import torch
+    y = reshaped_t2w
+    if not (_is_torch(y) and y.is_cuda and y.dtype == torch.float32 and y.is_contiguous() and y.dim() == 2):
+        raise ValueError("device input must be a contiguous float32 CUDA tensor [N, E]")
+    if y.device.index != _state["device"]:
+        raise ValueError(f"tensor on cuda:{y.device.index}, library bound to cuda:{_state['device']}")
+    if y.shape[1] != p.n_echo:
+        raise ValueError(f"reshaped_t2w has {y.shape[1]} echoes, TEeffs has {p.n_echo}")
+    idx = mask_indices
+    if idx is not None:
+        if not _is_torch(idx):
+            idx = np.asarray(idx)
+            idx = torch.as_tensor(np.ascontiguousarray(idx, dtype=np.int32 if idx.dtype == np.int32 else np.int64), device=y.device)
+        idx = idx.to(device=y.device, dtype=torch.int32 if idx.dtype == torch.int32 else torch.int64).contiguous()
+        p.idx_dtype = _abi.IDX_I32 if idx.dtype == torch.int32 else _abi.IDX_I64
+    p.echoes, p.memory, p.layout, p.ld = y.data_ptr(), _abi.MEM_DEVICE, _abi.LAYOUT_AOS, 0
+    p.mask_idx = idx.data_ptr() if idx is not None else None
+    p.n_vox, p.n_fit = y.shape[0], (y.shape[0] if idx is None else idx.numel())
+    return idx
 
 
 def fit_voxels_batch(reshaped_t2w, mask_indices, TEeffs, fit, fit_params, prior=True, norm=False, *,
@@ -398,20 +424,8 @@ def fit_voxels_batch(reshaped_t2w, mask_indices, TEeffs, fit, fit_params, prior=
     if dev:
         import torch
         y = reshaped_t2w
-        if not y.is_cuda or y.dtype != torch.float32 or not y.is_contiguous() or y.dim() != 2:
-            raise ValueError("device input must be a contiguous float32 CUDA tensor [N, E]")
-        if y.device.index != _state["device"]:
-            raise ValueError(f"tensor on cuda:{y.device.index}, library bound to cuda:{_state['device']}")
-        n_vox, n_echo = y.shape
-        idx = mask_indices
-        if idx is not None:
-            if not _is_torch(idx):
-                idx = np.asarray(idx)
-                idx = torch.as_tensor(np.ascontiguousarray(idx, dtype=np.int32 if idx.dtype == np.int32 else np.int64), device=y.device)
-            if idx.dtype not in (torch.int64, torch.int32) or not idx.is_contiguous():
-                idx = idx.to(torch.int64).contiguous()
-            p.idx_dtype = _abi.IDX_I32 if idx.dtype == torch.int32 else _abi.IDX_I64
-        m = n_vox if idx is None else idx.numel()
+        idx = _device_rows(p, y, mask_indices)
+        m = p.n_fit
 
         def alloc(dt=torch.float32):
             return torch.empty(m, dtype=dt, device=y.device)
@@ -424,8 +438,6 @@ def fit_voxels_batch(reshaped_t2w, mask_indices, TEeffs, fit, fit_params, prior=
             out["trace_f"] = torch.full((m, trace_cap), float("nan"), dtype=torch.float32, device=y.device)
             out["trace_step"] = torch.full((m, trace_cap), float("nan"), dtype=torch.float32, device=y.device)
             out["trace_len"] = torch.zeros(m, dtype=torch.int32, device=y.device)
-        p.echoes, p.memory = y.data_ptr(), _abi.MEM_DEVICE
-        p.mask_idx = idx.data_ptr() if idx is not None else None
         ptr = lambda t: t.data_ptr() if t is not None else None
         stream = torch.cuda.current_stream(y.device).cuda_stream
         dcnt = _device_counts(torch, y.device)
@@ -436,6 +448,8 @@ def fit_voxels_batch(reshaped_t2w, mask_indices, TEeffs, fit, fit_params, prior=
         if y.ndim != 2:
             raise ValueError("reshaped_t2w must be [N, E]")
         n_vox, n_echo = y.shape
+        if n_echo != p.n_echo:
+            raise ValueError(f"reshaped_t2w has {n_echo} echoes, TEeffs has {p.n_echo}")
         idx = None
         if mask_indices is not None:               # int32 indices are taken as they are (half the index bytes over PCIe)
             idx = np.asarray(mask_indices)
@@ -453,15 +467,13 @@ def fit_voxels_batch(reshaped_t2w, mask_indices, TEeffs, fit, fit_params, prior=
             out["trace_len"] = np.zeros(m, np.int32)
         p.echoes, p.memory = y.ctypes.data, _abi.MEM_HOST
         p.mask_idx = idx.ctypes.data if idx is not None else None
+        p.layout, p.ld, p.n_vox, p.n_fit = _abi.LAYOUT_AOS, 0, n_vox, m
         ptr = lambda a: a.ctypes.data if a is not None else None
         stream = None
         keep += [y, idx]
-    if n_echo != p.n_echo:
-        raise ValueError(f"reshaped_t2w has {n_echo} echoes, TEeffs has {p.n_echo}")
     if tracing:
         o.trace_f, o.trace_step, o.trace_len = ptr(out["trace_f"]), ptr(out["trace_step"]), ptr(out["trace_len"])
         o.trace_cap = int(trace_cap)
-    p.layout, p.ld, p.n_vox, p.n_fit = _abi.LAYOUT_AOS, 0, n_vox, m
     o.t2, o.k, o.res = ptr(out["t2"]), ptr(out["k"]), ptr(out["res"])
     o.sigma = ptr(out["sigma"]) if fit != "gaussian" else None
     o.fun, o.nit, o.status = ptr(out["fun"]), ptr(out["nit"]), ptr(out["status"])
@@ -470,14 +482,11 @@ def fit_voxels_batch(reshaped_t2w, mask_indices, TEeffs, fit, fit_params, prior=
     se = (None, None, None)
     if "se" in want:
         if dev:
-            se_t = torch.empty((3, m), dtype=torch.float32, device=y.device)
-            if m:
-                _stderr_launch(lib, p, fit, [ptr(out["k"]), ptr(out["t2"]), ptr(out["sigma"])], 0,
-                               [se_t[i].data_ptr() for i in range(3)], stream)
-            se = (se_t[0], se_t[1], se_t[2] if fit != "gaussian" else None)
+            se = _stderr_pass(lib, p, fit, out["k"], out["t2"], out["sigma"], False)
         else:
-            rows = y if idx is None else y[idx]
-            se = _stderr_staged(lib, p, fit, rows, out["k"], out["t2"], out["sigma"])
+            ps, (_, k, t2, sg) = _staged(p, y if idx is None else y[idx], out["k"], out["t2"], out["sigma"])
+            se = _stderr_pass(lib, ps, fit, k, t2, sg, True).cpu().numpy()
+        se = (se[0], se[1], se[2] if fit != "gaussian" else None)
     if dev:
         counts = None
         if check_bounds:                           # one small D2H: waits for the call (check_bounds=False stays asynchronous)
@@ -507,21 +516,10 @@ def fit_voxels_into(reshaped_t2w, mask_indices, TEeffs, fit, fit_params, prior, 
     p, o = _abi.Problem(), _abi.Outputs()
     keep = [_fill_problem(p, fit, fit_params, TEeffs, prior, norm, 0, 0.0, "auto", solver)]
     y = reshaped_t2w
-    if not (_is_torch(y) and y.is_cuda and y.dtype == torch.float32 and y.is_contiguous() and y.dim() == 2):
-        raise ValueError("device input must be a contiguous float32 CUDA tensor [N, E]")
-    idx = mask_indices
-    if idx is not None and not (_is_torch(idx) and idx.is_cuda and idx.dtype in (torch.int64, torch.int32) and idx.is_contiguous()):
-        idx = torch.as_tensor(np.ascontiguousarray(np.asarray(idx.cpu() if _is_torch(idx) else idx), dtype=np.int64), device=y.device)
-    if idx is not None:
-        p.idx_dtype = _abi.IDX_I32 if idx.dtype == torch.int32 else _abi.IDX_I64
+    idx = _device_rows(p, y, mask_indices)
     if counts is None:
         counts = _device_counts(torch, y.device)           # never the per-process counters: nothing leaks into later calls
     o.counts_dev = counts.data_ptr()
-    if y.shape[1] != p.n_echo:
-        raise ValueError(f"reshaped_t2w has {y.shape[1]} echoes, TEeffs has {p.n_echo}")
-    p.echoes, p.memory, p.layout = y.data_ptr(), _abi.MEM_DEVICE, _abi.LAYOUT_AOS
-    p.mask_idx = idx.data_ptr() if idx is not None else None
-    p.n_vox, p.n_fit = y.shape[0], (y.shape[0] if idx is None else idx.numel())
     o.t2, o.k, o.res = out["t2"], out["k"], out["res"]
     o.sigma = out.get("sigma") if fit != "gaussian" else None
     o.status, o.nit, o.fun = out.get("status"), out.get("nit"), out.get("fun")
@@ -622,32 +620,47 @@ def t2map_volume(t2w, mask, TEeffs, fit, fit_params, prior=True, norm=False, std
     out = tuple(maps[i].reshape(shape3) for i in range(4))
     if not stderr and t2_interval is None:
         return out
-    if stderr:
+    if stderr:                                     # (k, t2, sigma) rows of the pass, (t2, k, sigma) maps out
         if stream is not None:
-            se = torch.zeros((3, n_vox), dtype=torch.float32, device=y.device)
-            if m:
-                _stderr_launch(lib, p, fit, [mp[1], mp[0], mp[2]], 1, [se[1].data_ptr(), se[0].data_ptr(), se[2].data_ptr()], stream)
+            se = _stderr_pass(lib, p, fit, maps[1], maps[0], maps[2], True)
         else:
+            ps, (_, k, t2, sg) = _staged(p, y[idx], maps[1][idx], maps[0][idx], maps[2][idx])
             se = np.zeros((3, n_vox), np.float32)
-            sk, st, ss = _stderr_staged(lib, p, fit, y[idx], maps[1][idx], maps[0][idx], maps[2][idx])
-            se[0][idx], se[1][idx] = st, sk
-            if ss is not None:
-                se[2][idx] = ss
-        out = out + (tuple(se[i].reshape(shape3) for i in range(3)),)
+            se[:, idx] = _stderr_pass(lib, ps, fit, k, t2, sg, True).cpu().numpy()
+        out = out + (tuple(se[i].reshape(shape3) for i in (1, 0, 2)),)
     if t2_interval is not None:
         q, G = _interval_q(fit, n_echo, t2_interval), 64
         if stream is not None:
-            iv = torch.zeros((3, n_vox), dtype=torch.float32, device=y.device)
-            ivf = torch.zeros(n_vox, dtype=torch.uint8, device=y.device)
-            if m:
-                _interval_launch(lib, p, q, G, 1, [iv[0].data_ptr(), iv[1].data_ptr(), iv[2].data_ptr(), ivf.data_ptr()], None,
-                                 stream)
+            iv, ivf, _ = _interval_pass(lib, p, q, G, True, False, y.device)
         else:
-            iv = np.zeros((3, n_vox), np.float32)
-            ivf = np.zeros(n_vox, np.uint8)
-            iv[0][idx], iv[1][idx], iv[2][idx], ivf[idx], _ = _interval_staged(lib, p, y[idx], q, G, False)
+            ps, (ys,) = _staged(p, y[idx])
+            f, fl, _ = _interval_pass(lib, ps, q, G, True, False, ys.device)
+            iv, ivf = np.zeros((3, n_vox), np.float32), np.zeros(n_vox, np.uint8)
+            iv[:, idx], ivf[idx] = f.cpu().numpy(), fl.cpu().numpy()
         out = out + (tuple(iv[i].reshape(shape3) for i in range(3)) + (ivf.reshape(shape3),),)
     return out
+
+
+def _map_problem(reshaped_t2w, TEeffs, fit, norm, mask_indices, *maps):
+    """The device problem of a pass over existing maps: ``reshaped_t2w`` (float32), ``mask_indices`` (int64) and the
+    ``maps`` (float32, flattened) moved to the bound GPU, contiguous; TE, model and norm from the arguments, placeholder
+    fit parameters (these passes take none).  Returns (p, y, maps, keep); ``keep`` must stay alive for the call."""
+    import torch
+    dev = torch.device("cuda", _state["device"])
+
+    def to_dev(a, dt):
+        t = a if _is_torch(a) else torch.from_numpy(np.ascontiguousarray(a))
+        return t.to(device=dev, dtype=dt).contiguous()
+    y = to_dev(reshaped_t2w, torch.float32)
+    idx = to_dev(mask_indices, torch.int64)
+    maps = [to_dev(a, torch.float32).reshape(-1) for a in maps]
+    p = _abi.Problem()
+    dummy = {"initial_guess": [1.0, 100.0] + ([1.0] if fit != "gaussian" else []),
+             "param_bounds": [(0.0, 1e9), (1e-3, 1e9)] + ([(0.0, 1e9)] if fit != "gaussian" else [])}
+    te = _fill_problem(p, fit, dummy, TEeffs, True, norm, 0, 0.0, "loglinear")
+    p.echoes, p.memory, p.layout, p.mask_idx = y.data_ptr(), _abi.MEM_DEVICE, _abi.LAYOUT_AOS, idx.data_ptr()
+    p.n_vox, p.n_fit = y.shape[0], idx.numel()
+    return p, y, maps, (te, idx)
 
 
 def compute_residuals(reshaped_t2w, TEeffs, fit, norm, k_map, t2_map, sigma_map, res_map, mask_indices, mask):
@@ -656,28 +669,15 @@ def compute_residuals(reshaped_t2w, TEeffs, fit, norm, k_map, t2_map, sigma_map,
     stand-alone CUDA residual pass (``t2fit_residuals``); numpy inputs are staged through torch."""
     import torch
     lib = init()
-    dev = torch.device("cuda", _state["device"])
-    host = not _is_torch(reshaped_t2w)
-
-    def to_dev(a, dt):
-        t = a if _is_torch(a) else torch.from_numpy(np.ascontiguousarray(a))
-        return t.to(device=dev, dtype=dt).contiguous()
-    y = to_dev(reshaped_t2w, torch.float32)
-    idx = to_dev(mask_indices, torch.int64)
-    k, t2, sg = (to_dev(a, torch.float32).reshape(-1) for a in (k_map, t2_map, sigma_map))
-    res = to_dev(res_map, torch.float32).reshape(-1).clone()
-    p = _abi.Problem()
-    dummy = {"initial_guess": [1.0, 100.0] + ([1.0] if fit != "gaussian" else []),
-             "param_bounds": [(0.0, 1e9), (1e-3, 1e9)] + ([(0.0, 1e9)] if fit != "gaussian" else [])}
-    keep = _fill_problem(p, fit, dummy, TEeffs, True, norm, 0, 0.0, "loglinear")
-    p.echoes, p.memory, p.layout, p.mask_idx = y.data_ptr(), _abi.MEM_DEVICE, _abi.LAYOUT_AOS, idx.data_ptr()
-    p.n_vox, p.n_fit = y.shape[0], idx.numel()
-    stream = torch.cuda.current_stream(dev).cuda_stream
+    p, y, (k, t2, sg, res), keep = _map_problem(reshaped_t2w, TEeffs, fit, norm, mask_indices, k_map, t2_map, sigma_map,
+                                                res_map)
+    res = res.clone()
+    stream = torch.cuda.current_stream(y.device).cuda_stream
     _abi.check(lib, lib.t2fit_residuals(C.byref(p), k.data_ptr(), t2.data_ptr(), sg.data_ptr(), res.data_ptr(), stream),
                "t2fit_residuals")
     del keep
     shape3 = tuple(mask.shape[:3])
-    if host:
+    if not _is_torch(reshaped_t2w):
         return res.cpu().numpy().reshape(shape3)
     return res.reshape(shape3)
 
@@ -692,34 +692,16 @@ def parameter_stderr(reshaped_t2w, TEeffs, fit, norm, k_map, t2_map, sigma_map, 
     'gaussian_rician' ``sqrt(diag(s^2 (J'J)^-1))`` with ``s^2 = sum_e r_e^2 / (E - P)`` (scipy ``curve_fit``'s ``pcov``);
     for 'rician' ``sqrt(diag(H^-1))``, H the Hessian of the summed negative log-likelihood.  NaN where the voxel's input
     is not finite (rician: an echo <= 0), T2 <= 0, E <= P, or the matrix is not positive definite (DESIGN.md section 11)."""
-    import torch
     lib = init()
-    dev = torch.device("cuda", _state["device"])
-    host = not _is_torch(reshaped_t2w)
-
-    def to_dev(a, dt):
-        t = a if _is_torch(a) else torch.from_numpy(np.ascontiguousarray(a))
-        return t.to(device=dev, dtype=dt).contiguous()
-    y = to_dev(reshaped_t2w, torch.float32)
-    idx = to_dev(mask_indices, torch.int64)
-    k, t2, sg = (to_dev(a, torch.float32).reshape(-1) for a in (k_map, t2_map, sigma_map))
-    se = torch.zeros((3, y.shape[0]), dtype=torch.float32, device=dev)
-    p = _abi.Problem()
-    dummy = {"initial_guess": [1.0, 100.0] + ([1.0] if fit != "gaussian" else []),
-             "param_bounds": [(0.0, 1e9), (1e-3, 1e9)] + ([(0.0, 1e9)] if fit != "gaussian" else [])}
-    keep = _fill_problem(p, fit, dummy, TEeffs, True, norm, 0, 0.0, "loglinear")
+    p, y, (k, t2, sg), keep = _map_problem(reshaped_t2w, TEeffs, fit, norm, mask_indices, k_map, t2_map, sigma_map)
     if y.dim() != 2 or y.shape[1] != p.n_echo:
         raise ValueError(f"reshaped_t2w must be [N, {p.n_echo}]")
-    p.echoes, p.memory, p.layout, p.mask_idx = y.data_ptr(), _abi.MEM_DEVICE, _abi.LAYOUT_AOS, idx.data_ptr()
-    p.n_vox, p.n_fit = y.shape[0], idx.numel()
-    stream = torch.cuda.current_stream(dev).cuda_stream
-    _stderr_launch(lib, p, fit, [k.data_ptr(), t2.data_ptr(), sg.data_ptr()], 1,
-                   [se[1].data_ptr(), se[0].data_ptr(), se[2].data_ptr()], stream)
+    se = _stderr_pass(lib, p, fit, k, t2, sg, True)
     del keep
     shape3 = tuple(mask.shape[:3])
-    if host:
+    if not _is_torch(reshaped_t2w):
         se = se.cpu().numpy()
-    return tuple(se[i].reshape(shape3) for i in range(3))
+    return tuple(se[i].reshape(shape3) for i in (1, 0, 2))
 
 
 def t2_interval(reshaped_t2w, mask_indices, TEeffs, fit, fit_params, prior=True, norm=False, *, level=0.95, n_grid=64,
@@ -739,7 +721,6 @@ def t2_interval(reshaped_t2w, mask_indices, TEeffs, fit, fit_params, prior=True,
     determined), 4 the set is not one interval at grid resolution, 8 invalid (NaN; non-finite echoes, rician echoes <= 0,
     E <= P, the --no_prior voxel with S(TE0) above the k bound).  The interval does not depend on the fit's point, so it is
     the same whichever solver fits the maps.  ``n_grid``: 16..256 grid points (default 64)."""
-    import torch
     lib = init()
     p = _abi.Problem()
     keep = [_fill_problem(p, fit, fit_params, TEeffs, prior, norm, 0, 0.0, "auto")]
@@ -748,38 +729,15 @@ def t2_interval(reshaped_t2w, mask_indices, TEeffs, fit, fit_params, prior=True,
         raise ValueError("n_grid must lie in 16..256")
     t_lo, t_hi = (NO_PRIOR_T2_BOUNDS if not prior else (p.lb[1], p.ub[1]))
     if _is_torch(reshaped_t2w):
-        y = reshaped_t2w
-        if not y.is_cuda or y.dtype != torch.float32 or not y.is_contiguous() or y.dim() != 2:
-            raise ValueError("device input must be a contiguous float32 CUDA tensor [N, E]")
-        if y.device.index != _state["device"]:
-            raise ValueError(f"tensor on cuda:{y.device.index}, library bound to cuda:{_state['device']}")
-        if y.shape[1] != p.n_echo:
-            raise ValueError(f"reshaped_t2w has {y.shape[1]} echoes, TEeffs has {p.n_echo}")
-        idx = mask_indices
-        if idx is not None:
-            if not _is_torch(idx):
-                idx = np.asarray(idx)
-                idx = torch.as_tensor(np.ascontiguousarray(idx, dtype=np.int32 if idx.dtype == np.int32 else np.int64), device=y.device)
-            if idx.dtype not in (torch.int64, torch.int32) or not idx.is_contiguous():
-                idx = idx.to(torch.int64).contiguous()
-            p.idx_dtype = _abi.IDX_I32 if idx.dtype == torch.int32 else _abi.IDX_I64
-        m = y.shape[0] if idx is None else idx.numel()
-        f = torch.empty((3, m), dtype=torch.float32, device=y.device)
-        fl = torch.empty(m, dtype=torch.uint8, device=y.device)
-        pr = torch.empty((m, n_grid), dtype=torch.float64, device=y.device) if profile else None
-        p.echoes, p.memory, p.layout, p.ld = y.data_ptr(), _abi.MEM_DEVICE, _abi.LAYOUT_AOS, 0
-        p.mask_idx = idx.data_ptr() if idx is not None else None
-        p.n_vox, p.n_fit = y.shape[0], m
-        _interval_launch(lib, p, q, n_grid, 0, [f[0].data_ptr(), f[1].data_ptr(), f[2].data_ptr(), fl.data_ptr()],
-                         pr.data_ptr() if pr is not None else None, torch.cuda.current_stream(y.device).cuda_stream)
-        keep += [y, idx]
-        lo, hi, best = f[0], f[1], f[2]
+        keep += [_device_rows(p, reshaped_t2w, mask_indices)]
+        f, fl, pr = _interval_pass(lib, p, q, n_grid, False, profile, reshaped_t2w.device)
     else:
         y = np.asarray(reshaped_t2w)
         if y.ndim != 2 or y.shape[1] != p.n_echo:
             raise ValueError(f"reshaped_t2w must be [N, {p.n_echo}]")
-        rows = y if mask_indices is None else y[np.asarray(mask_indices)]
-        lo, hi, best, fl, pr = _interval_staged(lib, p, rows, q, n_grid, profile)
+        ps, (ys,) = _staged(p, y if mask_indices is None else y[np.asarray(mask_indices)])
+        f, fl, pr = (t.cpu().numpy() if t is not None else None for t in _interval_pass(lib, ps, q, n_grid, True, profile, ys.device))
+    lo, hi, best = f[0], f[1], f[2]
     del keep
     if not profile:
         return lo, hi, best, fl

@@ -16,6 +16,8 @@
 #pragma once
 #include <stdint.h>
 #include <math.h>
+#include <type_traits>
+#include <utility>
 
 #if defined(__CUDACC__) && !defined(T2FIT_HOSTSIM)
 #define T2_HD __device__ __forceinline__
@@ -28,6 +30,20 @@
 namespace t2fit {
 
 constexpr int kMaxEcho = 32;
+
+// Host-side echo-count dispatch: f(std::integral_constant<int, E>{}) for the run-time n_echo == E in 2..kMaxEcho, a
+// value-initialised result (nullptr for a kernel pointer) for any other count.  Every per-echo-count template table goes
+// through it, so this is the one place that decides which E are instantiated.
+template <class F, int... I>
+auto with_echo_count(int n_echo, F&& f, std::integer_sequence<int, I...>) {
+    decltype(f(std::integral_constant<int, 2>{})) r{};
+    ((n_echo == I + 2 ? (void)(r = f(std::integral_constant<int, I + 2>{})) : (void)0), ...);
+    return r;
+}
+template <class F>
+auto with_echo_count(int n_echo, F&& f) {
+    return with_echo_count(n_echo, f, std::make_integer_sequence<int, kMaxEcho - 1>{});
+}
 
 enum Model : int { kMono2 = 0, kFloor3 = 1 };
 enum Status : int { kOk = 0, kNonFinite = 1, kNotConverged = 2, kBadBounds = 3 };

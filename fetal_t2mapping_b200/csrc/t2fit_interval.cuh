@@ -23,7 +23,7 @@
 //   3. Bisection in log T2 of the two threshold crossings that bound the hull, to a width of kTolCross (the inside end is
 //      returned).  Off-grid points start from the fixed start and the solutions at the two enclosing grid points.
 //
-// Plain C++ when T2FIT_HOSTSIM is defined (tests/hostsim/interval_shim.cpp checks it against oracle/interval_oracle.py).
+// Plain C++ when T2FIT_HOSTSIM is defined (tests/hostsim/pass_shim.cpp checks it against oracle/interval_oracle.py).
 #pragma once
 #include "t2fit_stderr.cuh"
 

@@ -1017,31 +1017,46 @@ __global__ void __launch_bounds__(256) residual_kernel(const __grid_constant__ F
 }
 
 // ------------------------------------------------------------------------------------------------
-// stderr_kernel: per-voxel standard errors of (k, T2[, sigma]) at given parameters (t2fit_stderr, csrc/t2fit_stderr.cuh).
-// One thread per voxel, FP64; echoes read as the fit kernels read AoS rows (vector loads where E and the base allow).
+// Per-voxel analysis passes (t2fit_stderr, t2fit_t2_interval): one FP64 thread per voxel on AoS device rows, read as the fit
+// kernels read them (vector loads where E and the base allow).  PassInput is what both take from the problem.
 // ------------------------------------------------------------------------------------------------
-struct StderrArgs {
+struct PassInput {
     double te[kMaxEcho];
     const float* echoes;
     const int64_t* idx;        // at most one of idx / idx32 is set; neither = rows 0..n_fit-1
     const int32_t* idx32;
     int64_t n_fit, n_vox;
-    const float *k, *t2, *sigma;
-    float *se_k, *se_t2, *se_sigma;
-    int dense;                 // parameters and standard errors indexed by row instead of i
+    int dense;                 // outputs indexed by row instead of i
     int norm;
     int vec_ok;
+};
+
+struct PassSlot {
+    int64_t row;               // echo row of voxel i
+    int64_t o;                 // its output slot: row (dense) or i (compact)
+    bool in_range;             // row < n_vox
+};
+
+__device__ __forceinline__ PassSlot pass_slot(const PassInput& in, int64_t i) {
+    const int64_t row = in.idx ? __ldg(in.idx + i) : in.idx32 ? (int64_t)__ldg(in.idx32 + i) : i;
+    const bool in_range = (unsigned long long)row < (unsigned long long)in.n_vox;
+    return {row, in.dense ? row : i, in_range};
+}
+
+// stderr_kernel: standard errors of (k, T2[, sigma]) at given parameters (csrc/t2fit_stderr.cuh)
+struct StderrArgs {
+    PassInput in;
+    const float *k, *t2, *sigma;
+    float *se_k, *se_t2, *se_sigma;
 };
 
 template <int MODEL, int E>
 __global__ void __launch_bounds__(256) stderr_kernel(const __grid_constant__ StderrArgs a) {
     const int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x;
-    if (i >= a.n_fit) return;
-    const int64_t row = a.idx ? __ldg(a.idx + i) : a.idx32 ? (int64_t)__ldg(a.idx32 + i) : i;
-    const bool in_range = (unsigned long long)row < (unsigned long long)a.n_vox;
-    const int64_t o = a.dense ? row : i;
+    if (i >= a.in.n_fit) return;
+    const auto [row, o, in_range] = pass_slot(a.in, i);
     if (!in_range) {                        // an index outside the volume: nothing to read; a compact slot gets NaN
-        if (!a.dense) {
+        if (!a.in.dense) {
             if (a.se_k) a.se_k[o] = NAN;
             if (a.se_t2) a.se_t2[o] = NAN;
             if (MODEL != T2FIT_MODEL_GAUSSIAN && a.se_sigma) a.se_sigma[o] = NAN;
@@ -1049,9 +1064,9 @@ __global__ void __launch_bounds__(256) stderr_kernel(const __grid_constant__ Std
         return;
     }
     float y[E];
-    load_aos<E>(a.echoes, row, a.vec_ok, y);
+    load_aos<E>(a.in.echoes, row, a.in.vec_ok, y);
     double s[3];
-    se::voxel_stderr<MODEL, E>(y, a.te, a.norm != 0, __ldg(a.k + o), __ldg(a.t2 + o),
+    se::voxel_stderr<MODEL, E>(y, a.in.te, a.in.norm != 0, __ldg(a.k + o), __ldg(a.t2 + o),
                                MODEL == T2FIT_MODEL_GAUSSIAN ? 0.0f : __ldg(a.sigma + o), s);
     if (a.se_k) a.se_k[o] = (float)s[0];
     if (a.se_t2) a.se_t2[o] = (float)s[1];
@@ -1060,61 +1075,40 @@ __global__ void __launch_bounds__(256) stderr_kernel(const __grid_constant__ Std
 
 using StderrFn = void (*)(const StderrArgs);
 
-template <int MODEL>
-StderrFn pick_stderr_e(int n_echo) {
-    switch (n_echo) {
-#define T2_CASE(E) case E: return stderr_kernel<MODEL, E>;
-        T2_CASE(2) T2_CASE(3) T2_CASE(4) T2_CASE(5) T2_CASE(6) T2_CASE(7) T2_CASE(8) T2_CASE(9) T2_CASE(10)
-        T2_CASE(11) T2_CASE(12) T2_CASE(13) T2_CASE(14) T2_CASE(15) T2_CASE(16) T2_CASE(17) T2_CASE(18)
-        T2_CASE(19) T2_CASE(20) T2_CASE(21) T2_CASE(22) T2_CASE(23) T2_CASE(24) T2_CASE(25) T2_CASE(26)
-        T2_CASE(27) T2_CASE(28) T2_CASE(29) T2_CASE(30) T2_CASE(31) T2_CASE(32)
-#undef T2_CASE
-        default: return nullptr;
-    }
-}
-
 StderrFn pick_stderr(int model, int n_echo) {
-    if (model == T2FIT_MODEL_GAUSSIAN) return pick_stderr_e<T2FIT_MODEL_GAUSSIAN>(n_echo);
-    if (model == T2FIT_MODEL_GAUSSIAN_RICIAN) return pick_stderr_e<T2FIT_MODEL_GAUSSIAN_RICIAN>(n_echo);
-    if (model == T2FIT_MODEL_RICIAN) return pick_stderr_e<T2FIT_MODEL_RICIAN>(n_echo);
-    return nullptr;
+    return with_echo_count(n_echo, [model](auto e) -> StderrFn {
+        constexpr int E = decltype(e)::value;
+        if (model == T2FIT_MODEL_GAUSSIAN) return stderr_kernel<T2FIT_MODEL_GAUSSIAN, E>;
+        if (model == T2FIT_MODEL_GAUSSIAN_RICIAN) return stderr_kernel<T2FIT_MODEL_GAUSSIAN_RICIAN, E>;
+        if (model == T2FIT_MODEL_RICIAN) return stderr_kernel<T2FIT_MODEL_RICIAN, E>;
+        return nullptr;
+    });
 }
 
-// ------------------------------------------------------------------------------------------------
-// interval_kernel: per-voxel profile-likelihood interval for T2 (t2fit_t2_interval, csrc/t2fit_interval.cuh).
-// One thread per voxel, FP64.  The kernel is instantiated per echo count for the row load only; the model is a run-time
-// argument and the profile work is one out-of-line routine with E at run time, so its code is compiled 31 times rather than
-// 93 (ptxas gives every kernel its own copy of the routine).  The grid work space (iv::Grid, 6 KB) is thread-local memory.
-// ------------------------------------------------------------------------------------------------
+// interval_kernel: profile-likelihood interval for T2 (csrc/t2fit_interval.cuh).  The kernel is instantiated per echo count
+// for the row load only; the model is a run-time argument and the profile work is one out-of-line routine with E at run
+// time, so its code is compiled 31 times rather than 93 (ptxas gives every kernel its own copy of the routine).  The grid
+// work space (iv::Grid, 6 KB) is thread-local memory.
 struct IntervalArgs {
-    double te[kMaxEcho];
+    PassInput in;
     iv::Box box;               // k / T2 / sigma bounds in force; k_lo replaced by y(TE_0) per voxel when no_prior
     double q;
-    const float* echoes;
-    const int64_t* idx;        // at most one of idx / idx32 is set; neither = rows 0..n_fit-1
-    const int32_t* idx32;
-    int64_t n_fit, n_vox;
     float *lo, *hi, *best;
     uint8_t* flags;
     double* profile;           // [n_fit, n_grid] or NULL
     int model;
     int n_grid;
-    int dense;                 // lo / hi / best / flags indexed by row instead of i
-    int norm;
     int no_prior;
-    int vec_ok;
 };
 
 template <int E>
 __global__ void __launch_bounds__(128) interval_kernel(const __grid_constant__ IntervalArgs a) {
     const int64_t i = (int64_t)blockIdx.x * 128 + threadIdx.x;
-    if (i >= a.n_fit) return;
-    const int64_t row = a.idx ? __ldg(a.idx + i) : a.idx32 ? (int64_t)__ldg(a.idx32 + i) : i;
-    const bool in_range = (unsigned long long)row < (unsigned long long)a.n_vox;
-    const int64_t o = a.dense ? row : i;
+    if (i >= a.in.n_fit) return;
+    const auto [row, o, in_range] = pass_slot(a.in, i);
     double* prof = a.profile ? a.profile + i * a.n_grid : nullptr;
     if (!in_range) {                        // an index outside the volume: nothing to read; a compact slot gets NaN / invalid
-        if (!a.dense) {
+        if (!a.in.dense) {
             if (a.lo) a.lo[o] = NAN;
             if (a.hi) a.hi[o] = NAN;
             if (a.best) a.best[o] = NAN;
@@ -1124,10 +1118,10 @@ __global__ void __launch_bounds__(128) interval_kernel(const __grid_constant__ I
         return;
     }
     float y[E];
-    load_aos<E>(a.echoes, row, a.vec_ok, y);
+    load_aos<E>(a.in.echoes, row, a.in.vec_ok, y);
     iv::Voxel v;
     iv::Grid w;
-    const bool ok = iv::load_voxel<E>(y, a.te, a.model, a.norm != 0, a.box, a.no_prior != 0, v);
+    const bool ok = iv::load_voxel<E>(y, a.in.te, a.model, a.in.norm != 0, a.box, a.no_prior != 0, v);
     double lo, hi, best;
     int fl;
     iv::voxel_interval(v, ok, a.q, a.n_grid, w, lo, hi, best, fl, prof);
@@ -1140,15 +1134,7 @@ __global__ void __launch_bounds__(128) interval_kernel(const __grid_constant__ I
 using IntervalFn = void (*)(const IntervalArgs);
 
 IntervalFn pick_interval(int n_echo) {
-    switch (n_echo) {
-#define T2_CASE(E) case E: return interval_kernel<E>;
-        T2_CASE(2) T2_CASE(3) T2_CASE(4) T2_CASE(5) T2_CASE(6) T2_CASE(7) T2_CASE(8) T2_CASE(9) T2_CASE(10)
-        T2_CASE(11) T2_CASE(12) T2_CASE(13) T2_CASE(14) T2_CASE(15) T2_CASE(16) T2_CASE(17) T2_CASE(18)
-        T2_CASE(19) T2_CASE(20) T2_CASE(21) T2_CASE(22) T2_CASE(23) T2_CASE(24) T2_CASE(25) T2_CASE(26)
-        T2_CASE(27) T2_CASE(28) T2_CASE(29) T2_CASE(30) T2_CASE(31) T2_CASE(32)
-#undef T2_CASE
-        default: return nullptr;
-    }
+    return with_echo_count(n_echo, [](auto e) -> IntervalFn { return interval_kernel<decltype(e)::value>; });
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1158,15 +1144,7 @@ using FitFn = void (*)(const FitConsts, const KernelIO);
 
 template <int MODEL, int LAYOUT, bool FILL>
 FitFn pick_e(int n_echo) {
-    switch (n_echo) {
-#define T2_CASE(E) case E: return fit_kernel<MODEL, E, LAYOUT, FILL>;
-        T2_CASE(2) T2_CASE(3) T2_CASE(4) T2_CASE(5) T2_CASE(6) T2_CASE(7) T2_CASE(8) T2_CASE(9) T2_CASE(10)
-        T2_CASE(11) T2_CASE(12) T2_CASE(13) T2_CASE(14) T2_CASE(15) T2_CASE(16) T2_CASE(17) T2_CASE(18)
-        T2_CASE(19) T2_CASE(20) T2_CASE(21) T2_CASE(22) T2_CASE(23) T2_CASE(24) T2_CASE(25) T2_CASE(26)
-        T2_CASE(27) T2_CASE(28) T2_CASE(29) T2_CASE(30) T2_CASE(31) T2_CASE(32)
-#undef T2_CASE
-        default: return nullptr;
-    }
+    return with_echo_count(n_echo, [](auto e) -> FitFn { return fit_kernel<MODEL, decltype(e)::value, LAYOUT, FILL>; });
 }
 
 template <bool FILL>
@@ -1190,15 +1168,7 @@ using QueueFn = void (*)(const FitConsts, const KernelIO, unsigned long long*, c
 
 template <int LAYOUT>
 QueueFn pick_queue_e(int n_echo) {
-    switch (n_echo) {
-#define T2_CASE(E) case E: return floor_queue_kernel<E, LAYOUT>;
-        T2_CASE(2) T2_CASE(3) T2_CASE(4) T2_CASE(5) T2_CASE(6) T2_CASE(7) T2_CASE(8) T2_CASE(9) T2_CASE(10)
-        T2_CASE(11) T2_CASE(12) T2_CASE(13) T2_CASE(14) T2_CASE(15) T2_CASE(16) T2_CASE(17) T2_CASE(18)
-        T2_CASE(19) T2_CASE(20) T2_CASE(21) T2_CASE(22) T2_CASE(23) T2_CASE(24) T2_CASE(25) T2_CASE(26)
-        T2_CASE(27) T2_CASE(28) T2_CASE(29) T2_CASE(30) T2_CASE(31) T2_CASE(32)
-#undef T2_CASE
-        default: return nullptr;
-    }
+    return with_echo_count(n_echo, [](auto e) -> QueueFn { return floor_queue_kernel<decltype(e)::value, LAYOUT>; });
 }
 
 QueueFn pick_queue_kernel(int n_echo, int layout) {
@@ -1832,6 +1802,35 @@ int run_host(Context* c, const t2fit_problem& p, t2fit_outputs& o, const FitCons
     return T2FIT_OK;
 }
 
+// The checks t2fit_stderr and t2fit_t2_interval (`name`) make first, in this order, before their own.
+int check_pass_problem(const t2fit_problem* p, const char* name) {
+    if (!p) return fail(T2FIT_EINVAL, "NULL problem");
+    if (p->layout != T2FIT_LAYOUT_AOS) return fail(T2FIT_EINVAL, std::string(name) + " reads T2FIT_LAYOUT_AOS echoes only");
+    if (p->memory != T2FIT_MEM_DEVICE) return fail(T2FIT_EINVAL, std::string(name) + " takes T2FIT_MEM_DEVICE pointers only");
+    if (p->n_echo < 2 || p->n_echo > T2FIT_MAX_ECHO) return fail(T2FIT_EINVAL, "n_echo out of range (2..T2FIT_MAX_ECHO)");
+    if (p->model != T2FIT_MODEL_GAUSSIAN && p->model != T2FIT_MODEL_GAUSSIAN_RICIAN && p->model != T2FIT_MODEL_RICIAN)
+        return fail(T2FIT_EINVAL, "unknown model");
+    if (p->n_fit < 0 || p->n_vox < 0) return fail(T2FIT_EINVAL, "negative size");
+    if (p->idx_dtype != T2FIT_IDX_I64 && p->idx_dtype != T2FIT_IDX_I32) return fail(T2FIT_EINVAL, "bad idx_dtype");
+    if (!p->te_ms) return fail(T2FIT_EINVAL, "NULL te_ms");
+    return T2FIT_OK;
+}
+
+// The kernel input of a checked problem with n_fit > 0 and echoes set; n_fit > n_vox is each entry's last argument check.
+int pass_input(const t2fit_problem* p, int32_t dense, PassInput& in) {
+    if (!p->mask_idx && p->n_fit > p->n_vox) return fail(T2FIT_EINVAL, "n_fit > n_vox");
+    for (int e = 0; e < p->n_echo; ++e) in.te[e] = p->te_ms[e];
+    in.echoes = p->echoes;
+    if (p->mask_idx) {
+        if (p->idx_dtype == T2FIT_IDX_I32) in.idx32 = reinterpret_cast<const int32_t*>(p->mask_idx);
+        else in.idx = p->mask_idx;
+    }
+    in.n_fit = p->n_fit; in.n_vox = p->n_vox;
+    in.dense = dense != 0; in.norm = p->norm != 0;
+    in.vec_ok = (reinterpret_cast<uintptr_t>(p->echoes) % 16) == 0;
+    return T2FIT_OK;
+}
+
 }  // namespace
 
 // ================================================================================================
@@ -2368,30 +2367,13 @@ int t2fit_stderr(const t2fit_problem* p, const float* k, const float* t2, const 
                  float* se_t2, float* se_sigma, void* stream) {
     Context* c = g_ctx;
     if (!c) return fail(T2FIT_ENOTINIT, "t2fit_init() has not succeeded");
-    if (!p) return fail(T2FIT_EINVAL, "NULL problem");
-    if (p->layout != T2FIT_LAYOUT_AOS) return fail(T2FIT_EINVAL, "t2fit_stderr reads T2FIT_LAYOUT_AOS echoes only");
-    if (p->memory != T2FIT_MEM_DEVICE) return fail(T2FIT_EINVAL, "t2fit_stderr takes T2FIT_MEM_DEVICE pointers only");
-    if (p->n_echo < 2 || p->n_echo > T2FIT_MAX_ECHO) return fail(T2FIT_EINVAL, "n_echo out of range (2..T2FIT_MAX_ECHO)");
-    if (p->model != T2FIT_MODEL_GAUSSIAN && p->model != T2FIT_MODEL_GAUSSIAN_RICIAN && p->model != T2FIT_MODEL_RICIAN)
-        return fail(T2FIT_EINVAL, "unknown model");
-    if (p->n_fit < 0 || p->n_vox < 0) return fail(T2FIT_EINVAL, "negative size");
-    if (p->idx_dtype != T2FIT_IDX_I64 && p->idx_dtype != T2FIT_IDX_I32) return fail(T2FIT_EINVAL, "bad idx_dtype");
-    if (!p->te_ms) return fail(T2FIT_EINVAL, "NULL te_ms");
+    if (int rc = check_pass_problem(p, "t2fit_stderr")) return rc;
     if (p->n_fit == 0) return T2FIT_OK;
     if (!p->echoes || !k || !t2 || (p->model != T2FIT_MODEL_GAUSSIAN && !sigma)) return fail(T2FIT_EINVAL, "NULL echoes / parameters");
-    if (!p->mask_idx && p->n_fit > p->n_vox) return fail(T2FIT_EINVAL, "n_fit > n_vox");
     StderrArgs a{};
-    for (int e = 0; e < p->n_echo; ++e) a.te[e] = p->te_ms[e];
-    a.echoes = p->echoes;
-    if (p->mask_idx) {
-        if (p->idx_dtype == T2FIT_IDX_I32) a.idx32 = reinterpret_cast<const int32_t*>(p->mask_idx);
-        else a.idx = p->mask_idx;
-    }
-    a.n_fit = p->n_fit; a.n_vox = p->n_vox;
+    if (int rc = pass_input(p, dense, a.in)) return rc;
     a.k = k; a.t2 = t2; a.sigma = sigma;
     a.se_k = se_k; a.se_t2 = se_t2; a.se_sigma = se_sigma;
-    a.dense = dense != 0; a.norm = p->norm != 0;
-    a.vec_ok = (reinterpret_cast<uintptr_t>(p->echoes) % 16) == 0;
     const StderrFn fn = pick_stderr(p->model, p->n_echo);
     CU_TRY(cudaSetDevice(c->device));
     fn<<<(unsigned)((p->n_fit + 255) / 256), 256, 0, (cudaStream_t)stream>>>(a);
@@ -2403,15 +2385,7 @@ int t2fit_t2_interval(const t2fit_problem* p, double q, int32_t n_grid, int32_t 
                       float* t2_best, uint8_t* flags, double* profile, void* stream) {
     Context* c = g_ctx;
     if (!c) return fail(T2FIT_ENOTINIT, "t2fit_init() has not succeeded");
-    if (!p) return fail(T2FIT_EINVAL, "NULL problem");
-    if (p->layout != T2FIT_LAYOUT_AOS) return fail(T2FIT_EINVAL, "t2fit_t2_interval reads T2FIT_LAYOUT_AOS echoes only");
-    if (p->memory != T2FIT_MEM_DEVICE) return fail(T2FIT_EINVAL, "t2fit_t2_interval takes T2FIT_MEM_DEVICE pointers only");
-    if (p->n_echo < 2 || p->n_echo > T2FIT_MAX_ECHO) return fail(T2FIT_EINVAL, "n_echo out of range (2..T2FIT_MAX_ECHO)");
-    if (p->model != T2FIT_MODEL_GAUSSIAN && p->model != T2FIT_MODEL_GAUSSIAN_RICIAN && p->model != T2FIT_MODEL_RICIAN)
-        return fail(T2FIT_EINVAL, "unknown model");
-    if (p->n_fit < 0 || p->n_vox < 0) return fail(T2FIT_EINVAL, "negative size");
-    if (p->idx_dtype != T2FIT_IDX_I64 && p->idx_dtype != T2FIT_IDX_I32) return fail(T2FIT_EINVAL, "bad idx_dtype");
-    if (!p->te_ms) return fail(T2FIT_EINVAL, "NULL te_ms");
+    if (int rc = check_pass_problem(p, "t2fit_t2_interval")) return rc;
     if (n_grid < iv::kMinGrid || n_grid > iv::kMaxGrid) return fail(T2FIT_EINVAL, "n_grid out of range (16..256)");
     if (!(q >= 0.0) || !(q - q == 0.0)) return fail(T2FIT_EINVAL, "q must be finite and >= 0");
     iv::Box b{p->lb[0], p->ub[0], p->lb[1], p->ub[1], p->lb[2], p->ub[2]};
@@ -2422,20 +2396,12 @@ int t2fit_t2_interval(const t2fit_problem* p, double q, int32_t n_grid, int32_t 
     else if (!(b.s_lo > 0.0)) return fail(T2FIT_EINVAL, "the sigma lower bound must be > 0");
     if (p->n_fit == 0) return T2FIT_OK;
     if (!p->echoes) return fail(T2FIT_EINVAL, "NULL echoes");
-    if (!p->mask_idx && p->n_fit > p->n_vox) return fail(T2FIT_EINVAL, "n_fit > n_vox");
     IntervalArgs a{};
-    for (int e = 0; e < p->n_echo; ++e) a.te[e] = p->te_ms[e];
+    if (int rc = pass_input(p, dense, a.in)) return rc;
     a.box = b;
     a.q = q;
-    a.echoes = p->echoes;
-    if (p->mask_idx) {
-        if (p->idx_dtype == T2FIT_IDX_I32) a.idx32 = reinterpret_cast<const int32_t*>(p->mask_idx);
-        else a.idx = p->mask_idx;
-    }
-    a.n_fit = p->n_fit; a.n_vox = p->n_vox;
     a.lo = t2_lo; a.hi = t2_hi; a.best = t2_best; a.flags = flags; a.profile = profile;
-    a.model = p->model; a.n_grid = n_grid; a.dense = dense != 0; a.norm = p->norm != 0; a.no_prior = p->no_prior != 0;
-    a.vec_ok = (reinterpret_cast<uintptr_t>(p->echoes) % 16) == 0;
+    a.model = p->model; a.n_grid = n_grid; a.no_prior = p->no_prior != 0;
     const IntervalFn fn = pick_interval(p->n_echo);
     CU_TRY(cudaSetDevice(c->device));
     fn<<<(unsigned)((p->n_fit + 127) / 128), 128, 0, (cudaStream_t)stream>>>(a);

@@ -12,7 +12,7 @@
 // of A is <= 0, or a Cholesky pivot is <= 0 or not finite; otherwise they are finite and >= 0 (0 only for a least-squares
 // fit with every residual exactly zero), however ill-determined the voxel.
 //
-// Plain C++ when T2FIT_HOSTSIM is defined (tests/hostsim/stderr_shim.cpp checks it against oracle/stderr_oracle.py).
+// Plain C++ when T2FIT_HOSTSIM is defined (tests/hostsim/pass_shim.cpp checks it against oracle/stderr_oracle.py).
 #pragma once
 #include "../../include/t2fit.h"
 #include "t2fit_lbfgsb.cuh"

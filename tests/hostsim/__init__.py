@@ -18,18 +18,24 @@ DEPS = [SRC] + [os.path.join(HERE, "..", "..", "fetal_t2mapping_b200", "csrc", f
 SO_STRICT = os.path.join(HERE, "libt2fit_hostsim_strict.so")
 
 
-def build(force=False, strict=False):
-    """strict=False: -mfma + contraction, as the device fuses a*b+c (cancellation noise, e.g. D - k*C at a converged point,
+def compile_so(src, so, deps, force=False, strict=False):
+    """g++ ``src`` into the shared library ``so`` unless it is newer than every file of ``deps``.
+    strict=False: -mfma + contraction, as the device fuses a*b+c (cancellation noise, e.g. D - k*C at a converged point,
     is then as small on the host simulation as on the GPU).  strict=True: no contraction at all -- every product and sum
     rounds separately whatever the expression shape, so two implementations that perform the same operations in the same
     order agree BIT FOR BIT (the serial and the cooperative L-BFGS-B solver, tests/test_hostsim_coop.py)."""
-    so = SO_STRICT if strict else SO
-    if not force and os.path.isfile(so) and all(os.path.getmtime(so) >= os.path.getmtime(d) for d in DEPS):
+    if not force and os.path.isfile(so) and all(os.path.getmtime(so) >= os.path.getmtime(d) for d in deps):
         return so
     fp = ["-ffp-contract=off"] if strict else ["-mfma", "-ffp-contract=fast"]
-    cmd = ["g++", "-O2", "-std=c++17"] + fp + ["-shared", "-fPIC", "-x", "c++", SRC, "-o", so, "-lm"]
+    tmp = f"{so[:-3]}.{os.getpid()}.tmp.so"
+    cmd = ["g++", "-O2", "-std=c++17"] + fp + ["-shared", "-fPIC", "-x", "c++", src, "-o", tmp, "-lm"]
     subprocess.run(cmd, check=True, cwd=HERE)
+    os.replace(tmp, so)    # test processes that build at once (the ranks of a distributed test) never load a partial file
     return so
+
+
+def build(force=False, strict=False):
+    return compile_so(SRC, SO_STRICT if strict else SO, DEPS, force, strict)
 
 
 _libs = {}

@@ -112,6 +112,11 @@ def test_entries_agree_and_nothing_else_moves(gpu_lib, fit, solver, device):
     valid = (fl & 8) == 0
     assert valid.mean() > (0.9 if fit != "rician" else 0.0)
     assert np.all(lo[valid] <= best[valid]) and np.all(best[valid] <= hi[valid])
+    if device:                                     # an index tensor in host memory is moved to the echoes' GPU
+        for dt in (torch.int64, torch.int32):
+            got = gpu_lib.t2_interval(cv(flat), torch.from_numpy(idx).to(dt), te, fit, fp, prior=False, norm=False)
+            for a, b in zip(got, (lo, hi, best, fl)):
+                assert np.array_equal(_np(a), b, equal_nan=True)
 
 
 # The three scenarios of test_gpu_stderr.py::test_standard_error_is_calibrated (32 echoes at TE = 10..320 ms, bounds far

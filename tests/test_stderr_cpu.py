@@ -10,7 +10,7 @@ from scipy.special import i1e
 from oracle import stderr_oracle as so
 from oracle.fit_oracle import model_floor, model_mono, objective_rician_nll
 from tests.conftest import load_golden
-from tests.hostsim import stderr_shim
+from tests.hostsim import pass_shim as stderr_shim
 
 FIXTURES = ["c1_gaussian_noprior", "c1_gaussian_prior", "c2_gaussian_noprior", "c2_gaussian_hf_prior", "c4_gaussian_noprior",
             "c3_floor_noprior", "c3_floor_prior", "c5_floor_noprior", "c3_rician_prior", "norm_gaussian",
