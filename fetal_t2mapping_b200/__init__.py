@@ -7,9 +7,9 @@ else of the reference (DICOM->BIDS, registration, segmentation, NIfTI I/O, plots
 reference.  There is no CPU implementation of the fit in this package.
 """
 from .presets import preset, set_fit_params                                           # noqa: F401
-from .api import (FitResult, compute_residuals, device_info, fit_voxels_batch, init,   # noqa: F401
-                  mask_indices_device, parameter_stderr, pinned_array, shutdown, t2_interval, t2map_volume,
-                  work_model)
+from .api import (BootstrapMaps, BootstrapResult, FitResult, compute_residuals,      # noqa: F401
+                  device_info, fit_voxels_batch, init, mask_indices_device, parameter_stderr, parametric_bootstrap,
+                  pinned_array, shutdown, t2_interval, t2map_volume, work_model)
 
 from .roi import phantom_roi_table, roi_stats, save_phantom_csv, set_phantom_gt        # noqa: F401
 from .loader import VolumeMaps, t2map_series                                          # noqa: F401

@@ -128,6 +128,10 @@ SYMBOLS = [
                                C.c_void_p, C.c_void_p]),
     ("t2fit_t2_interval", C.c_int, [C.POINTER(Problem), C.c_double, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p,
                                     C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
+    ("t2fit_bootstrap_replicates", C.c_int, [C.POINTER(Problem), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                             C.c_uint64, C.c_int32, C.c_void_p, C.c_void_p]),
+    ("t2fit_bootstrap_stats", C.c_int, [C.c_int32, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                        C.c_double] + [C.c_void_p] * 7),
     ("t2fit_work_model", C.c_int, [C.c_int32, C.c_int32] + [C.POINTER(C.c_double)] * 5),
 ]
 

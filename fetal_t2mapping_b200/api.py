@@ -18,6 +18,7 @@ from __future__ import annotations
 
 import ctypes as C
 import os
+from collections import namedtuple
 from dataclasses import dataclass
 
 import numpy as np
@@ -26,7 +27,8 @@ from . import _abi
 from .presets import NO_PRIOR_K_UB, NO_PRIOR_T2_BOUNDS
 
 __all__ = ["fit_voxels_batch", "fit_voxels_into", "check_counts", "t2map_volume", "compute_residuals", "parameter_stderr", "t2_interval", "FitResult", "init",
-           "shutdown", "device_info", "mask_indices_device", "work_model", "pinned_array", "BOUNDS_ERROR"]
+           "parametric_bootstrap", "BootstrapResult", "BootstrapMaps", "shutdown", "device_info", "mask_indices_device",
+           "work_model", "pinned_array", "BOUNDS_ERROR"]
 
 BOUNDS_ERROR = "An upper bound is less than the corresponding lower bound."   # scipy's text
 
@@ -503,18 +505,20 @@ def fit_voxels_batch(reshaped_t2w, mask_indices, TEeffs, fit, fit_params, prior=
                      out.get("trace_len"), *se)
 
 
-def fit_voxels_into(reshaped_t2w, mask_indices, TEeffs, fit, fit_params, prior, norm, out, *, solver="auto", counts=None):
+def fit_voxels_into(reshaped_t2w, mask_indices, TEeffs, fit, fit_params, prior, norm, out, *, solver="auto", counts=None,
+                    init_mode="auto", max_iter=0, tol=0.0):
     """Device-memory fit whose compact results go to caller-given raw device pointers: ``out`` maps 't2', 'k', 'res'
     (and 'sigma' for the 3-parameter fits; optionally 'status', 'nit', 'fun') to integer addresses of arrays with room
     for ``len(mask_indices)`` elements -- local memory or a peer GPU's buffer mapped with ``t2fit_shared_open`` (the
-    fused gather of ``distributed.fit_voxels_sharded``).  Asynchronous on the current torch stream.  ``counts``: a zeroed
-    int64 CUDA tensor [4] the call adds its histogram to (slot 0 indices out of range, 1..3 voxels per non-OK status);
-    the caller reads it when it synchronises and raises as :func:`fit_voxels_batch` does (``check_counts``)."""
+    fused gather of ``distributed.fit_voxels_sharded``); an address may be None (that output is skipped).  Asynchronous on
+    the current torch stream.  ``counts``: a zeroed int64 CUDA tensor [4] the call adds its histogram to (slot 0 indices
+    out of range, 1..3 voxels per non-OK status); the caller reads it when it synchronises and raises as
+    :func:`fit_voxels_batch` does (``check_counts``).  ``init_mode``, ``max_iter``, ``tol`` as in :func:`fit_voxels_batch`."""
     import torch
     lib = init()
     solver = resolve_solver(fit, solver)
     p, o = _abi.Problem(), _abi.Outputs()
-    keep = [_fill_problem(p, fit, fit_params, TEeffs, prior, norm, 0, 0.0, "auto", solver)]
+    keep = [_fill_problem(p, fit, fit_params, TEeffs, prior, norm, max_iter, tol, init_mode, solver)]
     y = reshaped_t2w
     idx = _device_rows(p, y, mask_indices)
     if counts is None:
@@ -556,7 +560,8 @@ def mask_indices_device(mask, n_masks=None):
     return idx[:n.value]
 
 
-def t2map_volume(t2w, mask, TEeffs, fit, fit_params, prior=True, norm=False, stderr=False, t2_interval=None, **kw):
+def t2map_volume(t2w, mask, TEeffs, fit, fit_params, prior=True, norm=False, stderr=False, t2_interval=None, bootstrap=None,
+                 **kw):
     """Stacked per-TE volumes ``t2w[z,y,x,E]``, mask ``[z,y,x]`` or per-TE masks ``[z,y,x,E]`` and the
     TE vector in; ``(t2_map, k_map, sigma_map, res_map)`` float32 ``[z,y,x]`` out, zeros off-mask --
     the whole hot block of ``process_t2maps`` (run_t2mapping.py:383-386, :411-461, :471-473).
@@ -564,7 +569,9 @@ def t2map_volume(t2w, mask, TEeffs, fit, fit_params, prior=True, norm=False, std
     parameters (:func:`parameter_stderr`), float32 ``[z,y,x]``, zeros off-mask (se_sigma all zeros for 'gaussian').
     ``t2_interval=level`` (e.g. 0.95) appends ``(t2_lo_map, t2_hi_map, t2_best_map, flags_map)`` as the last element: the
     profile-likelihood confidence interval for T2 at that level (:func:`t2_interval`, default grid), float32 / uint8
-    ``[z,y,x]``, zeros off-mask."""
+    ``[z,y,x]``, zeros off-mask.  ``bootstrap=n_rep`` appends, after those, a :data:`BootstrapMaps` ``(t2_mean, t2_sd, t2_lo,
+    t2_hi, k_sd, sigma_sd, n_used, n_ok)`` of ``[z,y,x]`` maps, zeros off-mask: the parametric bootstrap of the fitted maps
+    (:func:`parametric_bootstrap` with level 0.95, seed 0 and the estimated noise level)."""
     lib = init()
     shape3 = tuple(t2w.shape[:3])
     n_echo = t2w.shape[-1]
@@ -618,7 +625,9 @@ def t2map_volume(t2w, mask, TEeffs, fit, fit_params, prior=True, norm=False, std
     elif o.status_count[3] > 0:
         raise ValueError(BOUNDS_ERROR)
     out = tuple(maps[i].reshape(shape3) for i in range(4))
-    if not stderr and t2_interval is None:
+    if bootstrap is not None:
+        _bootstrap_args(bootstrap, 0.95)
+    if not stderr and t2_interval is None and bootstrap is None:
         return out
     if stderr:                                     # (k, t2, sigma) rows of the pass, (t2, k, sigma) maps out
         if stream is not None:
@@ -638,6 +647,27 @@ def t2map_volume(t2w, mask, TEeffs, fit, fit_params, prior=True, norm=False, std
             iv, ivf = np.zeros((3, n_vox), np.float32), np.zeros(n_vox, np.uint8)
             iv[:, idx], ivf[idx] = f.cpu().numpy(), fl.cpu().numpy()
         out = out + (tuple(iv[i].reshape(shape3) for i in range(3)) + (ivf.reshape(shape3),),)
+    if bootstrap is not None:                      # compact (k, t2, sigma) of the fit; the noise keyed by the flat index
+        args = (fit, fit_params, TEeffs, prior, norm, solver, kw.get("init_mode", "auto"), kw.get("max_iter", 0),
+                kw.get("tol", 0.0))
+        sg = (lambda a: a) if fit != "gaussian" else (lambda a: None)
+        if stream is not None:
+            bs = _bootstrap_pass(lib, p, *args, [maps[1][idx], maps[0][idx], sg(maps[2][idx])], None, None, bootstrap, 0.95,
+                                 0, None)
+            new = lambda t: torch.zeros(n_vox, dtype=t.dtype, device=y.device).index_copy_(0, idx, t)
+        else:
+            import torch
+            ps, (_, k, t2, s) = _staged(p, y[idx], maps[1][idx], maps[0][idx], sg(maps[2][idx]))
+            bs = _bootstrap_pass(lib, ps, *args, [k, t2, s], None, torch.from_numpy(idx).to(k.device), bootstrap, 0.95, 0,
+                                 None)
+
+            def new(t):
+                a = np.zeros(n_vox, dtype=t.cpu().numpy().dtype)
+                a[idx] = t.cpu().numpy()
+                return a
+        mean, sd, lo, hi, nu, no = bs
+        cols = (mean[1], sd[1], lo, hi, sd[0], sd[2] if fit != "gaussian" else torch.zeros_like(sd[2]), nu, no)
+        out = out + (BootstrapMaps(*[new(c).reshape(shape3) for c in cols]),)
     return out
 
 
@@ -742,3 +772,171 @@ def t2_interval(reshaped_t2w, mask_indices, TEeffs, fit, fit_params, prior=True,
     if not profile:
         return lo, hi, best, fl
     return lo, hi, best, fl, pr, interval_grid(t_lo, t_hi, n_grid)
+
+
+@dataclass
+class BootstrapResult:
+    """Per-voxel parametric bootstrap (:func:`parametric_bootstrap`), compact over the fitted voxels.
+
+    ``mean``, ``sd``      float32 [M, P]  mean and standard deviation (ddof 1) of the refitted parameters, in the order of
+                                          ``FitResult.results`` (k, T2[, sigma])
+    ``t2_lo``, ``t2_hi``  float32 [M]     T2 quantiles at (1 - level) / 2 and (1 + level) / 2 of the refits
+    ``n_used``            int32 [M]       replicates whose refit has status 0 or 2 and finite parameters
+    ``n_ok``              int32 [M]       replicates whose refit has status 0
+    mean, sd, t2_lo and t2_hi are NaN where n_used < 2.  numpy for numpy input, CUDA tensors for CUDA input.
+    """
+    mean: object
+    sd: object
+    t2_lo: object
+    t2_hi: object
+    n_used: object
+    n_ok: object
+
+
+# the bootstrap maps t2map_volume(..., bootstrap=n_rep) appends: float32 [z,y,x] (n_used / n_ok int32), zeros off-mask
+BootstrapMaps = namedtuple("BootstrapMaps", "t2_mean t2_sd t2_lo t2_hi k_sd sigma_sd n_used n_ok")
+
+BOOTSTRAP_BUDGET = 1 << 30       # bytes of replicate rows plus refit results one chunk of voxels may hold
+
+
+def _bootstrap_chunk(n_echo, n_rep, fit):
+    """Voxels per chunk of the bootstrap: the replicate rows (float32 [n_rep, E]) and refit results (k, T2[, sigma] float32,
+    status uint8) of one voxel, within BOOTSTRAP_BUDGET."""
+    per_voxel = n_rep * (4 * n_echo + 4 * (2 if fit == "gaussian" else 3) + 1)
+    return max(1, BOOTSTRAP_BUDGET // per_voxel)
+
+
+def _bootstrap_pass(lib, p, fit, fit_params, TEeffs, prior, norm, solver, init_mode, max_iter, tol, params, noise, vid,
+                    n_rep, level, seed, chunk):
+    """The bootstrap of the device rows of ``p`` (AoS, compact): ``params`` (k, t2, sigma) float32 CUDA [M] (sigma None for
+    'gaussian'), ``noise`` float32 CUDA [M] or None, ``vid`` int64 CUDA [M] flat voxel ids or None (= the row read).  Per
+    chunk of voxels: t2fit_bootstrap_replicates into one replicate buffer, the refit by fit_voxels_into (same solver, preset,
+    prior and norm; status 3 is excluded by the statistics, never raised), t2fit_bootstrap_stats.  Asynchronous on the
+    current stream.  Returns float32 mean [3, M], sd [3, M], lo [M], hi [M] and int32 n_used [M], n_ok [M]."""
+    import torch
+    dev = params[0].device
+    M, E = p.n_fit, p.n_echo
+    P = 2 if fit == "gaussian" else 3
+    if p.mask_idx is None and vid is None:       # chunks read rows a.. of the echoes: key the noise by the row itself
+        vid = torch.arange(M, dtype=torch.int64, device=dev)
+    chunk = max(1, min(int(chunk) if chunk is not None else _bootstrap_chunk(E, n_rep, fit), M or 1))
+    mean, sd = torch.empty((3, M), dtype=torch.float32, device=dev), torch.empty((3, M), dtype=torch.float32, device=dev)
+    lo, hi = torch.empty(M, dtype=torch.float32, device=dev), torch.empty(M, dtype=torch.float32, device=dev)
+    nu, no = torch.empty(M, dtype=torch.int32, device=dev), torch.empty(M, dtype=torch.int32, device=dev)
+    rows = torch.empty((chunk * n_rep, E), dtype=torch.float32, device=dev)
+    rep = torch.empty((P, chunk * n_rep), dtype=torch.float32, device=dev)
+    rst = torch.empty(chunk * n_rep, dtype=torch.uint8, device=dev)
+    cm, cs = torch.empty(3 * chunk, dtype=torch.float32, device=dev), torch.empty(3 * chunk, dtype=torch.float32, device=dev)
+    counts = _device_counts(torch, dev)                      # the refit's histogram: status 3 is a replicate outcome here
+    stream = torch.cuda.current_stream(dev).cuda_stream
+    isz = 4 if p.idx_dtype == _abi.IDX_I32 else 8
+    ptr = lambda t, a: t[a:].data_ptr() if t is not None else None
+    out = {"t2": rep[1].data_ptr(), "k": rep[0].data_ptr(), "sigma": rep[2].data_ptr() if P == 3 else None, "res": None,
+           "status": rst.data_ptr()}
+    for a in range(0, M, chunk):
+        n = min(chunk, M - a)
+        q = _abi.Problem.from_buffer_copy(p)
+        q.n_fit = n
+        if p.mask_idx is not None:
+            q.mask_idx = p.mask_idx + a * isz
+        else:
+            q.echoes, q.n_vox = p.echoes + a * E * 4, p.n_vox - a
+        _abi.check(lib, lib.t2fit_bootstrap_replicates(C.byref(q), ptr(params[0], a), ptr(params[1], a), ptr(params[2], a),
+                                                       ptr(noise, a), ptr(vid, a), int(seed) & 0xFFFFFFFFFFFFFFFF,
+                                                       int(n_rep), rows.data_ptr(), stream), "t2fit_bootstrap_replicates")
+        fit_voxels_into(rows[:n * n_rep], None, TEeffs, fit, fit_params, prior, norm, out, solver=solver, counts=counts,
+                        init_mode=init_mode, max_iter=max_iter, tol=tol)
+        _abi.check(lib, lib.t2fit_bootstrap_stats(p.model, n, int(n_rep), rep[0].data_ptr(), rep[1].data_ptr(),
+                                                  rep[2].data_ptr() if P == 3 else None, rst.data_ptr(), float(level),
+                                                  cm.data_ptr(), cs.data_ptr(), ptr(lo, a), ptr(hi, a), ptr(nu, a), ptr(no, a),
+                                                  stream), "t2fit_bootstrap_stats")
+        mean[:, a:a + n] = cm[:3 * n].view(3, n)
+        sd[:, a:a + n] = cs[:3 * n].view(3, n)
+    return mean, sd, lo, hi, nu, no
+
+
+def _bootstrap_args(n_rep, level):
+    if not 16 <= int(n_rep) <= 4096:
+        raise ValueError("n_rep must lie in 16..4096")
+    if not 0.0 < float(level) < 1.0:
+        raise ValueError("level must lie in (0, 1)")
+
+
+def parametric_bootstrap(reshaped_t2w, mask_indices, TEeffs, fit, fit_params, prior=True, norm=False, *, n_rep=200,
+                         level=0.95, seed=0, noise_sd=None, params=None, solver="auto", init_mode="auto", chunk=None):
+    """Parametric bootstrap of the fit of every voxel ``mask_indices[i]`` of ``reshaped_t2w`` (float32 ``[N, E]``;
+    ``mask_indices`` None = all rows), with the arguments of :func:`fit_voxels_batch`: the sampling distribution of the
+    estimator as it is run -- solver, preset, bounds, early stopping, ``prior`` and ``norm`` included.
+
+    Per voxel: ``n_rep`` (16..4096) replicates are simulated from the fitted curve (DESIGN.md section 13) --
+    'gaussian' ``k u + s z``, 'gaussian_rician' ``sqrt((k u)^2 + sigma^2) + s z``, 'rician' the modulus of ``k u`` plus
+    complex noise of sd sigma_n, ``u = exp(-TE / T2)`` -- and refitted with the same solver.  ``s`` is ``noise_sd`` if
+    given (a float or an [M] array, in the units of the stored echoes) else ``sqrt(sum r^2 / (E - P))`` at the fit;
+    sigma_n is ``noise_sd`` if given else the fitted sigma.  The normals come from Philox4x32-10 keyed by ``seed`` and the
+    flat voxel index, so a voxel's replicates do not depend on which other voxels are bootstrapped or how they are chunked.
+    ``params``: the fit ``(k, t2, sigma)`` compact over the voxels (e.g. maps read back from NIfTI; sigma None for
+    'gaussian'); None fits first with ``solver`` / ``init_mode`` (raising what :func:`fit_voxels_batch` raises).  ``chunk``:
+    voxels per replicate buffer (default: 1 GiB of replicate rows plus refit results).
+
+    Returns a :class:`BootstrapResult`.  Replicates whose refit has status 1 or 3 are not used (an invalid voxel -- echoes
+    not finite, T2 <= 0, E <= P with s estimated -- gets NaN rows, so none of its replicates is used).  numpy input gives
+    numpy output (the masked rows are staged through torch); a CUDA tensor gives CUDA tensors, asynchronously on the
+    current stream when ``params`` is given."""
+    import torch
+    lib = init()
+    _bootstrap_args(n_rep, level)
+    solver = resolve_solver(fit, solver)
+    p = _abi.Problem()
+    keep = [_fill_problem(p, fit, fit_params, TEeffs, prior, norm, 0, 0.0, init_mode, solver)]
+    if params is None:
+        r = fit_voxels_batch(reshaped_t2w, mask_indices, TEeffs, fit, fit_params, prior, norm, solver=solver,
+                             init_mode=init_mode, want=("status",))
+        params = (r.k, r.t2, r.sigma if fit != "gaussian" else None)
+    if len(params) != 3:
+        raise ValueError("params must be (k, t2, sigma)")
+    dev_in = _is_torch(reshaped_t2w)
+    if dev_in:
+        keep += [_device_rows(p, reshaped_t2w, mask_indices)]
+        device = reshaped_t2w.device
+        vid, q = None, p
+        to_dev = lambda a: (a if _is_torch(a) else torch.from_numpy(np.ascontiguousarray(a))).to(
+            device=device, dtype=torch.float32).reshape(-1).contiguous()
+        par = [to_dev(a) if a is not None else None for a in params]
+    else:
+        y = np.asarray(reshaped_t2w)
+        if y.ndim != 2 or y.shape[1] != p.n_echo:
+            raise ValueError(f"reshaped_t2w must be [N, {p.n_echo}]")
+        ids = np.arange(y.shape[0], dtype=np.int64) if mask_indices is None else np.asarray(mask_indices).astype(np.int64)
+        if ids.size and (ids.min() < 0 or ids.max() >= y.shape[0]):
+            raise IndexError("mask_indices out of range")
+        host = lambda a: np.asarray(a.cpu() if _is_torch(a) else a)
+        q, (ys, *par) = _staged(p, y[ids], *[host(a) if a is not None else None for a in params])
+        device = ys.device
+        vid = torch.from_numpy(ids).to(device)
+        keep += [ys]
+        to_dev = lambda a: torch.from_numpy(np.ascontiguousarray(a, dtype=np.float32).reshape(-1)).to(device)
+    M = q.n_fit
+    if fit == "gaussian":
+        par[2] = None
+    elif par[2] is None:
+        raise ValueError(f"fit {fit!r} needs sigma in params")
+    if any(a is not None and a.numel() != M for a in par):
+        raise ValueError(f"params must hold {M} values each")
+    noise = None
+    if noise_sd is not None:
+        if np.ndim(noise_sd) == 0 and not _is_torch(noise_sd):
+            noise = torch.full((M,), float(noise_sd), dtype=torch.float32, device=device)
+        else:
+            noise = to_dev(noise_sd.cpu().numpy() if (_is_torch(noise_sd) and not dev_in) else noise_sd)
+            if noise.numel() != M:
+                raise ValueError(f"noise_sd must be a float or hold {M} values")
+    res = _bootstrap_pass(lib, q, fit, fit_params, TEeffs, prior, norm, solver, init_mode, 0, 0.0, par, noise, vid, n_rep,
+                          level, seed, chunk)
+    del keep
+    P = 2 if fit == "gaussian" else 3
+    mean, sd, lo, hi, nu, no = res
+    mean, sd = mean[:P].t().contiguous(), sd[:P].t().contiguous()
+    out = (mean, sd, lo, hi, nu, no)
+    if not dev_in:
+        out = tuple(t.cpu().numpy() for t in out)
+    return BootstrapResult(*out)

@@ -9,7 +9,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(CSRC, os.environ.get("T2FIT_LIB_NAME", "libt2fit.so"))   # T2FIT_LIB_NAME: variant builds for A/B runs
 SOURCES = ["t2fit_kernels.cu"]
-HEADERS = ["t2fit_core.cuh", "t2fit_lbfgsb.cuh", "t2fit_lbfgsb_coop.cuh", "t2fit_lbfgsb_dense.cuh", "t2fit_i0e_coeffs.h", "t2fit_i1e_coeffs.h", "t2fit_stderr.cuh", "t2fit_interval.cuh", "t2fit_consts.h", "t2fit_workers.h", os.path.join("..", "..", "include", "t2fit.h")]
+HEADERS = ["t2fit_core.cuh", "t2fit_lbfgsb.cuh", "t2fit_lbfgsb_coop.cuh", "t2fit_lbfgsb_dense.cuh", "t2fit_i0e_coeffs.h", "t2fit_i1e_coeffs.h", "t2fit_stderr.cuh", "t2fit_interval.cuh", "t2fit_bootstrap.cuh", "t2fit_consts.h", "t2fit_workers.h", os.path.join("..", "..", "include", "t2fit.h")]
 
 # No `--split-compile`: nvcc's parallel split compilation (rounds 1-2 used `--split-compile 0`, 70 s instead of 140 s) is NOT
 # reproducible -- two builds of the same sources gave libraries of 17.8 and 19.6 MB with different SASS for the same kernel

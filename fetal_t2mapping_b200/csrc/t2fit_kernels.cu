@@ -42,6 +42,7 @@
 #include "t2fit_lbfgsb_dense.cuh"
 #include "t2fit_stderr.cuh"
 #include "t2fit_interval.cuh"
+#include "t2fit_bootstrap.cuh"
 #include "t2fit_workers.h"
 
 using namespace t2fit;
@@ -1135,6 +1136,154 @@ using IntervalFn = void (*)(const IntervalArgs);
 
 IntervalFn pick_interval(int n_echo) {
     return with_echo_count(n_echo, [](auto e) -> IntervalFn { return interval_kernel<decltype(e)::value>; });
+}
+
+// replicate_kernel: the parametric-bootstrap rows of every voxel (csrc/t2fit_bootstrap.cuh).  One thread per (voxel,
+// replicate): thread g writes row g = i n_rep + r, so consecutive threads store consecutive rows.  The threads of a voxel
+// read the same observed row (served by L1) and recompute its source; the model is a run-time argument.
+struct ReplicateArgs {
+    PassInput in;
+    const float *k, *t2, *sigma;
+    const float* noise_sd;     // [n_fit] or NULL
+    const int64_t* voxel_id;   // [n_fit] or NULL = the row read
+    uint64_t seed;
+    float* rows;               // [n_fit * n_rep, E]
+    int n_rep;
+    int model;
+};
+
+template <int E>
+__global__ void __launch_bounds__(128) replicate_kernel(const __grid_constant__ ReplicateArgs a) {
+    const int64_t g = (int64_t)blockIdx.x * 128 + threadIdx.x;
+    if (g >= a.in.n_fit * a.n_rep) return;
+    const int64_t i = g / a.n_rep;
+    const int r = (int)(g - i * a.n_rep);
+    const auto [row, o, in_range] = pass_slot(a.in, i);
+    bs::Source<E> src;
+    src.ok = false;
+    if (in_range) {
+        float y[E];
+        load_aos<E>(a.in.echoes, row, a.in.vec_ok, y);
+        bs::load_source<E>(y, a.in.te, a.model, a.in.norm != 0, __ldg(a.k + i), __ldg(a.t2 + i),
+                           a.model == T2FIT_MODEL_GAUSSIAN ? 0.0f : __ldg(a.sigma + i), a.noise_sd != nullptr,
+                           a.noise_sd ? __ldg(a.noise_sd + i) : 0.0f, src);
+    }
+    const uint64_t v = a.voxel_id ? (uint64_t)__ldg(a.voxel_id + i) : (uint64_t)row;
+    float out[E];
+    bs::replicate_row<E>(src, a.model, a.seed, r, v, out);
+    float* dst = a.rows + g * E;
+#pragma unroll
+    for (int e = 0; e < E; ++e) dst[e] = out[e];
+}
+
+using ReplicateFn = void (*)(const ReplicateArgs);
+
+ReplicateFn pick_replicate(int n_echo) {
+    return with_echo_count(n_echo, [](auto e) -> ReplicateFn { return replicate_kernel<decltype(e)::value>; });
+}
+
+// bootstrap_stats_kernel: one block of kStatThreads per voxel.  Thread t sums the used replicates t, t + kStatThreads, ...
+// in ascending order, a halving tree adds the partial sums (the fixed order of csrc/t2fit_bootstrap.cuh), and a bitonic
+// sort of the used T2 values (unused slots +inf, padded to a power of two) in shared memory gives the quantiles.
+struct BootstrapStatsArgs {
+    const float *k, *t2, *sigma;
+    const uint8_t* status;
+    float *mean, *sd;          // [3][n_fit]
+    float *lo, *hi;
+    int32_t *n_used, *n_ok;
+    int64_t n_fit;
+    double q_lo, q_hi;
+    int n_rep, n_pad;          // n_pad: the power of two >= n_rep the sort runs over
+    int model;
+};
+
+__global__ void __launch_bounds__(bs::kStatThreads) bootstrap_stats_kernel(const __grid_constant__ BootstrapStatsArgs a) {
+    constexpr int T = bs::kStatThreads;
+    extern __shared__ float key[];                 // [n_pad]
+    __shared__ double part[3][T];
+    __shared__ int cnt[2][T];
+    const int t = threadIdx.x;
+    const int64_t i = blockIdx.x;
+    const int P = a.model == T2FIT_MODEL_GAUSSIAN ? 2 : 3;
+    const float* rk = a.k + i * a.n_rep;
+    const float* rt = a.t2 + i * a.n_rep;
+    const float* rs = P == 3 ? a.sigma + i * a.n_rep : nullptr;
+    const uint8_t* st = a.status + i * a.n_rep;
+    double s[3] = {0.0, 0.0, 0.0};
+    int nu = 0, no = 0;
+    for (int r = t; r < a.n_pad; r += T) {
+        float kt = INFINITY;
+        if (r < a.n_rep) {
+            const float vk = rk[r], vt = rt[r], vs = rs ? rs[r] : 0.0f;
+            const uint8_t sr = st[r];
+            no += sr == T2FIT_ST_OK;
+            if (bs::rep_used(sr, vk, vt, vs, P)) {
+                ++nu;
+                kt = vt;
+                s[0] = lb::add(s[0], (double)vk);
+                s[1] = lb::add(s[1], (double)vt);
+                if (P == 3) s[2] = lb::add(s[2], (double)vs);
+            }
+        }
+        key[r] = kt;
+    }
+    for (int j = 0; j < 3; ++j) part[j][t] = s[j];
+    cnt[0][t] = nu;
+    cnt[1][t] = no;
+    __syncthreads();
+    for (int h = T / 2; h >= 1; h /= 2) {
+        if (t < h) {
+            for (int j = 0; j < 3; ++j) part[j][t] = lb::add(part[j][t], part[j][t + h]);
+            cnt[0][t] += cnt[0][t + h];
+            cnt[1][t] += cnt[1][t + h];
+        }
+        __syncthreads();
+    }
+    const int n_used = cnt[0][0], n_ok = cnt[1][0];
+    double m[3];
+    for (int j = 0; j < 3; ++j) m[j] = part[j][0] / (double)n_used;
+    __syncthreads();                               // everyone has read the sums before part[] is reused
+    s[0] = s[1] = s[2] = 0.0;
+    for (int r = t; r < a.n_rep; r += T) {
+        const float vk = rk[r], vt = rt[r], vs = rs ? rs[r] : 0.0f;
+        if (!bs::rep_used(st[r], vk, vt, vs, P)) continue;
+        const double dk = lb::sub((double)vk, m[0]), dt = lb::sub((double)vt, m[1]);
+        s[0] = lb::add(s[0], lb::mul(dk, dk));
+        s[1] = lb::add(s[1], lb::mul(dt, dt));
+        if (P == 3) {
+            const double ds = lb::sub((double)vs, m[2]);
+            s[2] = lb::add(s[2], lb::mul(ds, ds));
+        }
+    }
+    for (int j = 0; j < 3; ++j) part[j][t] = s[j];
+    __syncthreads();
+    for (int h = T / 2; h >= 1; h /= 2) {
+        if (t < h)
+            for (int j = 0; j < 3; ++j) part[j][t] = lb::add(part[j][t], part[j][t + h]);
+        __syncthreads();
+    }
+    for (int size = 2; size <= a.n_pad; size *= 2) {          // bitonic sort, ascending
+        for (int stride = size / 2; stride > 0; stride /= 2) {
+            for (int x = t; x < a.n_pad / 2; x += T) {
+                const int lo = 2 * x - (x & (stride - 1)), hi = lo + stride;
+                const bool up = (lo & size) == 0;
+                const float u = key[lo], w = key[hi];
+                if ((u > w) == up) { key[lo] = w; key[hi] = u; }
+            }
+            __syncthreads();
+        }
+    }
+    if (t != 0) return;
+    const bool enough = n_used >= 2;
+    for (int j = 0; j < 3; ++j) {
+        const bool has = enough && j < P;
+        if (a.mean) a.mean[j * a.n_fit + i] = has ? (float)m[j] : NAN;
+        if (a.sd) a.sd[j * a.n_fit + i] = has ? (float)sqrt(part[j][0] / (double)(n_used - 1)) : NAN;
+    }
+    if (a.lo) a.lo[i] = enough ? (float)bs::quantile_sorted(key, n_used, a.q_lo) : NAN;
+    if (a.hi) a.hi[i] = enough ? (float)bs::quantile_sorted(key, n_used, a.q_hi) : NAN;
+    if (a.n_used) a.n_used[i] = n_used;
+    if (a.n_ok) a.n_ok[i] = n_ok;
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -2405,6 +2554,60 @@ int t2fit_t2_interval(const t2fit_problem* p, double q, int32_t n_grid, int32_t 
     const IntervalFn fn = pick_interval(p->n_echo);
     CU_TRY(cudaSetDevice(c->device));
     fn<<<(unsigned)((p->n_fit + 127) / 128), 128, 0, (cudaStream_t)stream>>>(a);
+    CU_TRY(cudaGetLastError());
+    return T2FIT_OK;
+}
+
+int t2fit_bootstrap_replicates(const t2fit_problem* p, const float* k, const float* t2, const float* sigma,
+                               const float* noise_sd, const int64_t* voxel_id, uint64_t seed, int32_t n_rep, float* rows,
+                               void* stream) {
+    Context* c = g_ctx;
+    if (!c) return fail(T2FIT_ENOTINIT, "t2fit_init() has not succeeded");
+    if (int rc = check_pass_problem(p, "t2fit_bootstrap_replicates")) return rc;
+    if (n_rep < bs::kMinRep || n_rep > bs::kMaxRep) return fail(T2FIT_EINVAL, "n_rep out of range (16..4096)");
+    if (p->n_fit == 0) return T2FIT_OK;
+    if (!p->echoes || !k || !t2 || (p->model != T2FIT_MODEL_GAUSSIAN && !sigma) || !rows)
+        return fail(T2FIT_EINVAL, "NULL echoes / parameters / rows");
+    if (p->n_fit > INT64_MAX / n_rep) return fail(T2FIT_EINVAL, "n_fit * n_rep overflows");
+    ReplicateArgs a{};
+    if (int rc = pass_input(p, 0, a.in)) return rc;
+    a.k = k; a.t2 = t2; a.sigma = sigma; a.noise_sd = noise_sd; a.voxel_id = voxel_id;
+    a.seed = seed; a.rows = rows; a.n_rep = n_rep; a.model = p->model;
+    const ReplicateFn fn = pick_replicate(p->n_echo);
+    const int64_t n = p->n_fit * n_rep;
+    if ((n + 127) / 128 > INT32_MAX) return fail(T2FIT_EINVAL, "n_fit * n_rep too large for one launch");
+    CU_TRY(cudaSetDevice(c->device));
+    fn<<<(unsigned)((n + 127) / 128), 128, 0, (cudaStream_t)stream>>>(a);
+    CU_TRY(cudaGetLastError());
+    return T2FIT_OK;
+}
+
+int t2fit_bootstrap_stats(int32_t model, int64_t n_fit, int32_t n_rep, const float* rep_k, const float* rep_t2,
+                          const float* rep_sigma, const uint8_t* rep_status, double level, float* mean, float* sd,
+                          float* t2_lo, float* t2_hi, int32_t* n_used, int32_t* n_ok, void* stream) {
+    Context* c = g_ctx;
+    if (!c) return fail(T2FIT_ENOTINIT, "t2fit_init() has not succeeded");
+    if (model != T2FIT_MODEL_GAUSSIAN && model != T2FIT_MODEL_GAUSSIAN_RICIAN && model != T2FIT_MODEL_RICIAN)
+        return fail(T2FIT_EINVAL, "unknown model");
+    if (n_fit < 0) return fail(T2FIT_EINVAL, "negative size");
+    if (n_rep < bs::kMinRep || n_rep > bs::kMaxRep) return fail(T2FIT_EINVAL, "n_rep out of range (16..4096)");
+    if (!(level > 0.0 && level < 1.0)) return fail(T2FIT_EINVAL, "level must lie in (0, 1)");
+    if (n_fit == 0) return T2FIT_OK;
+    if (!rep_k || !rep_t2 || !rep_status || (model != T2FIT_MODEL_GAUSSIAN && !rep_sigma))
+        return fail(T2FIT_EINVAL, "NULL replicate results");
+    if (n_fit > INT32_MAX) return fail(T2FIT_EINVAL, "n_fit too large for one launch");
+    BootstrapStatsArgs a{};
+    a.k = rep_k; a.t2 = rep_t2; a.sigma = rep_sigma; a.status = rep_status;
+    a.mean = mean; a.sd = sd; a.lo = t2_lo; a.hi = t2_hi; a.n_used = n_used; a.n_ok = n_ok;
+    a.n_fit = n_fit;
+    a.q_lo = 0.5 * (1.0 - level);
+    a.q_hi = 0.5 * (1.0 + level);
+    a.n_rep = n_rep;
+    a.n_pad = 1;
+    while (a.n_pad < n_rep) a.n_pad *= 2;
+    a.model = model;
+    CU_TRY(cudaSetDevice(c->device));
+    bootstrap_stats_kernel<<<(unsigned)n_fit, bs::kStatThreads, a.n_pad * sizeof(float), (cudaStream_t)stream>>>(a);
     CU_TRY(cudaGetLastError());
     return T2FIT_OK;
 }

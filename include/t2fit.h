@@ -309,6 +309,42 @@ int t2fit_stderr(const t2fit_problem *p, const float *k, const float *t2, const 
 int t2fit_t2_interval(const t2fit_problem *p, double q, int32_t n_grid, int32_t dense, float *t2_lo, float *t2_hi,
                       float *t2_best, uint8_t *flags, double *profile, void *stream);
 
+/* Per-voxel parametric bootstrap (DESIGN.md section 13, csrc/t2fit_bootstrap.cuh): simulate n_rep noisy replicates of every
+ * voxel from its fitted curve, refit them with t2fit_run (same problem: solver, init, x0 / bounds / options, no_prior, norm),
+ * and summarise the refitted parameters.  The two passes below bracket that refit.
+ *
+ * t2fit_bootstrap_replicates: for voxel i with the float32 parameters k[i], t2[i] (, sigma[i]) and the fit's echoes y (float32,
+ * scaled by y / max(y) in float32 when p->norm), rows[(i n_rep + r) n_echo + e] = replicate r, echo e, u_e = exp(-te_e / T2):
+ *   gaussian         k u_e + s z_e                          s = noise_sd[i] if given, else sqrt(sum_e r_e^2 / (E - P)) at
+ *   gaussian_rician  sqrt((k u_e)^2 + sigma^2) + s z_e        the parameters (FP64, as t2fit_stderr's s)
+ *   rician           sqrt((k u_e + sn z_2e)^2 + (sn z_2e+1)^2)   sn = noise_sd[i] if given, else sigma[i]
+ * FP64, stored as float32.  A given noise_sd is in the units of the stored echoes (divided by max(y) under norm).  z: standard
+ * normals from Philox4x32-10, key (seed lo32, seed hi32), counter (j, r, v lo32, v hi32), v = voxel_id[i] if given, else the
+ * row read (mask_idx[i], or i without an index); each word w gives u = (w + 0.5) 2^-32 and block j gives z_4j..z_4j+3 by
+ * Box-Muller on (w0, w1), (w2, w3): sqrt(-2 ln u_a) (cos 2 pi u_b, sin 2 pi u_b).  The rows of a voxel are all NaN (every
+ * refit gets status 1) when its index is outside [0, n_vox), an echo is not finite (rician: or <= 0), a parameter is not
+ * finite or T2 <= 0, the noise level is not finite or < 0, or E <= P with s to estimate.
+ * Reads echoes / layout / memory / mask_idx / idx_dtype / n_vox / n_fit / n_echo / te_ms / model / norm of *p; T2FIT_LAYOUT_AOS
+ * and T2FIT_MEM_DEVICE only.  k, t2, sigma (3-parameter models), noise_sd, voxel_id: device [n_fit] compact (element i =
+ * voxel mask_idx[i]), noise_sd / voxel_id may be NULL.  rows: device [n_fit * n_rep, n_echo].  Asynchronous on `stream`.
+ *
+ * t2fit_bootstrap_stats: for voxel i, replicate r at element i n_rep + r of rep_k / rep_t2 / rep_sigma / rep_status (the
+ * compact outputs of the refit; rep_sigma unused for gaussian): a replicate is used when its status is 0 or 2 and its
+ * parameters are finite.  n_used[i] = used replicates, n_ok[i] = replicates with status 0; mean[j n_fit + i] / sd[j n_fit + i]
+ * = FP64 mean / standard deviation (ddof 1) of parameter j = (k, T2, sigma) over the used replicates; t2_lo / t2_hi = the T2
+ * quantiles at (1 - level) / 2 and (1 + level) / 2 (numpy.quantile's default linear method).  NaN when n_used < 2, and for
+ * sigma of gaussian.  Sums run in a fixed order: deterministic.  Any output may be NULL (skipped).  Device pointers,
+ * asynchronous on `stream`.
+ *
+ * EINVAL: n_rep outside 16..4096, level outside (0, 1), NULL inputs, and the checks of t2fit_stderr; ENOTINIT before
+ * t2fit_init.  n_fit == 0 is a no-op. */
+int t2fit_bootstrap_replicates(const t2fit_problem *p, const float *k, const float *t2, const float *sigma,
+                               const float *noise_sd, const int64_t *voxel_id, uint64_t seed, int32_t n_rep, float *rows,
+                               void *stream);
+int t2fit_bootstrap_stats(int32_t model, int64_t n_fit, int32_t n_rep, const float *rep_k, const float *rep_t2,
+                          const float *rep_sigma, const uint8_t *rep_status, double level, float *mean, float *sd,
+                          float *t2_lo, float *t2_hi, int32_t *n_used, int32_t *n_ok, void *stream);
+
 /* Algorithmic work of the shipped kernels, for roofline accounting (DESIGN.md): FLOPs and MUFU ops
  * of one pass over the echoes, and the fixed per-voxel part. */
 int t2fit_work_model(int32_t model, int32_t n_echo, double *flop_per_pass, double *mufu_per_pass,
