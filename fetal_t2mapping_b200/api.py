@@ -361,16 +361,16 @@ def _interval_launch(lib, p, q, n_grid, dense, outs, profile, stream):
     _abi.check(lib, lib.t2fit_t2_interval(C.byref(p), q, int(n_grid), int(dense), *outs, profile, stream), "t2fit_t2_interval")
 
 
-def _interval_pass(lib, p, q, n_grid, dense, profile, device):
-    """t2fit_t2_interval on the device rows of ``p`` on the current stream of ``device``.  Returns (f, flags, prof): f
-    float32 [3, n] (lo, hi, best), flags uint8 [n] -- n = p.n_vox, zeros off the index, when ``dense``, else p.n_fit --
-    and with ``profile`` p at the grid, float64 [p.n_fit, n_grid], else None."""
+def _interval_pass(lib, p, q, n_grid, profile):
+    """t2fit_t2_interval on the device rows of ``p`` on the current stream of the bound GPU, compact.  Returns (f, flags,
+    prof): f float32 [3, p.n_fit] (lo, hi, best), flags uint8 [p.n_fit] and with ``profile`` p at the grid, float64
+    [p.n_fit, n_grid], else None."""
     import torch
-    new, n = (torch.zeros, p.n_vox) if dense else (torch.empty, p.n_fit)
-    f = new((3, n), dtype=torch.float32, device=device)
-    fl = new(n, dtype=torch.uint8, device=device)
+    device = torch.device("cuda", _state["device"])
+    f = torch.empty((3, p.n_fit), dtype=torch.float32, device=device)
+    fl = torch.empty(p.n_fit, dtype=torch.uint8, device=device)
     pr = torch.empty((p.n_fit, n_grid), dtype=torch.float64, device=device) if profile else None
-    _interval_launch(lib, p, q, n_grid, dense, [f[0].data_ptr(), f[1].data_ptr(), f[2].data_ptr(), fl.data_ptr()],
+    _interval_launch(lib, p, q, n_grid, 0, [f[0].data_ptr(), f[1].data_ptr(), f[2].data_ptr(), fl.data_ptr()],
                      pr.data_ptr() if pr is not None else None, torch.cuda.current_stream(device).cuda_stream)
     return f, fl, pr
 
@@ -399,6 +399,45 @@ def _device_rows(p, reshaped_t2w, mask_indices):
     p.mask_idx = idx.data_ptr() if idx is not None else None
     p.n_vox, p.n_fit = y.shape[0], (y.shape[0] if idx is None else idx.numel())
     return idx
+
+
+def _pass_input(p, reshaped_t2w, mask_indices, *params):
+    """The input of a pass over the voxels ``mask_indices`` (None = every row) of ``reshaped_t2w`` [N, E] for a problem ``p``
+    that :func:`_fill_problem` filled.  Returns (q, params, ids, fin, keep): ``q`` the device problem the pass entries read;
+    each per-voxel array of ``params`` as a contiguous float32 CUDA tensor [M] (None stays None); ``ids`` the int64 flat
+    voxel ids of q's rows (numpy) when q reads staged rows, None when it reads the echoes through the index; ``fin`` turns a
+    device result into what the caller returns (numpy for host input); ``keep`` must stay alive for the pass.  A CUDA tensor
+    is taken as :func:`_device_rows` takes it.  Host input: an index outside [0, N) raises IndexError, as in the fit; the
+    masked rows and the params are staged once (:func:`_staged`)."""
+    import torch
+    if _is_torch(reshaped_t2w):
+        idx = _device_rows(p, reshaped_t2w, mask_indices)
+        dev = reshaped_t2w.device
+        to_dev = lambda a: (a if _is_torch(a) else torch.from_numpy(np.ascontiguousarray(a))).to(
+            device=dev, dtype=torch.float32).reshape(-1).contiguous()
+        return p, [to_dev(a) if a is not None else None for a in params], None, (lambda t: t), [idx]
+    y = np.asarray(reshaped_t2w)
+    if y.ndim != 2 or y.shape[1] != p.n_echo:
+        raise ValueError(f"reshaped_t2w must be [N, {p.n_echo}]")
+    ids = np.arange(y.shape[0], dtype=np.int64) if mask_indices is None else np.asarray(mask_indices).astype(np.int64)
+    if ids.size and (ids.min() < 0 or ids.max() >= y.shape[0]):
+        raise IndexError("mask_indices out of range")
+    host = lambda a: a.cpu().numpy() if _is_torch(a) else a
+    q, (ys, *par) = _staged(p, y if mask_indices is None else y[ids], *[host(a) if a is not None else None for a in params])
+    return q, par, ids, (lambda t: t.cpu().numpy() if t is not None else None), [ys]
+
+
+def _scatter(vals, idx, n_vox):
+    """Compact values [..., M] of a pass (a CUDA tensor) for the flat voxels ``idx`` as [..., n_vox] of their dtype, zeros
+    elsewhere: a CUDA tensor for a CUDA ``idx``, else a numpy array."""
+    if _is_torch(idx):
+        import torch
+        return torch.zeros(tuple(vals.shape[:-1]) + (n_vox,), dtype=vals.dtype, device=vals.device).index_copy_(
+            vals.dim() - 1, idx, vals)
+    v = vals.cpu().numpy()
+    a = np.zeros(v.shape[:-1] + (n_vox,), dtype=v.dtype)
+    a[..., idx] = v
+    return a
 
 
 def fit_voxels_batch(reshaped_t2w, mask_indices, TEeffs, fit, fit_params, prior=True, norm=False, *,
@@ -483,11 +522,9 @@ def fit_voxels_batch(reshaped_t2w, mask_indices, TEeffs, fit, fit_params, prior=
     _run(lib, p, o, stream)
     se = (None, None, None)
     if "se" in want:
-        if dev:
-            se = _stderr_pass(lib, p, fit, out["k"], out["t2"], out["sigma"], False)
-        else:
-            ps, (_, k, t2, sg) = _staged(p, y if idx is None else y[idx], out["k"], out["t2"], out["sigma"])
-            se = _stderr_pass(lib, ps, fit, k, t2, sg, True).cpu().numpy()
+        ps, (k, t2, sg), _, fin, pin = _pass_input(p, y, idx, out["k"], out["t2"], out["sigma"])
+        keep += pin
+        se = fin(_stderr_pass(lib, ps, fit, k, t2, sg, False))
         se = (se[0], se[1], se[2] if fit != "gaussian" else None)
     if dev:
         counts = None
@@ -579,6 +616,9 @@ def t2map_volume(t2w, mask, TEeffs, fit, fit_params, prior=True, norm=False, std
     solver = resolve_solver(fit, kw.get("solver", "auto"))
     keep = [_fill_problem(p, fit, fit_params, TEeffs, prior, norm, kw.get("max_iter", 0), kw.get("tol", 0.0),
                           kw.get("init_mode", "auto"), solver)]
+    q = _interval_q(fit, p.n_echo, t2_interval) if t2_interval is not None else None
+    if bootstrap is not None:
+        _bootstrap_args(bootstrap, 0.95)
     fused_mask = None
     if _is_torch(t2w):
         import torch
@@ -625,49 +665,34 @@ def t2map_volume(t2w, mask, TEeffs, fit, fit_params, prior=True, norm=False, std
     elif o.status_count[3] > 0:
         raise ValueError(BOUNDS_ERROR)
     out = tuple(maps[i].reshape(shape3) for i in range(4))
-    if bootstrap is not None:
-        _bootstrap_args(bootstrap, 0.95)
     if not stderr and t2_interval is None and bootstrap is None:
         return out
+    import torch
+    # every pass runs compact over the masked voxels, on the fitted problem (device input) or on the masked rows staged once
+    if stream is not None:
+        ps, (t2, k, sg) = p, maps[:3].index_select(1, idx)
+    else:
+        ps, (ys, t2, k, sg) = _staged(p, y[idx], *maps[:3, idx])
+        keep.append(ys)
+    put = lambda t: _scatter(t, idx, n_vox)
     if stderr:                                     # (k, t2, sigma) rows of the pass, (t2, k, sigma) maps out
-        if stream is not None:
-            se = _stderr_pass(lib, p, fit, maps[1], maps[0], maps[2], True)
-        else:
-            ps, (_, k, t2, sg) = _staged(p, y[idx], maps[1][idx], maps[0][idx], maps[2][idx])
-            se = np.zeros((3, n_vox), np.float32)
-            se[:, idx] = _stderr_pass(lib, ps, fit, k, t2, sg, True).cpu().numpy()
+        se = _stderr_pass(lib, ps, fit, k, t2, sg, False)
+        if fit == "gaussian":
+            se[2].zero_()                          # left unset by the compact pass
+        se = put(se)
         out = out + (tuple(se[i].reshape(shape3) for i in (1, 0, 2)),)
     if t2_interval is not None:
-        q, G = _interval_q(fit, n_echo, t2_interval), 64
-        if stream is not None:
-            iv, ivf, _ = _interval_pass(lib, p, q, G, True, False, y.device)
-        else:
-            ps, (ys,) = _staged(p, y[idx])
-            f, fl, _ = _interval_pass(lib, ps, q, G, True, False, ys.device)
-            iv, ivf = np.zeros((3, n_vox), np.float32), np.zeros(n_vox, np.uint8)
-            iv[:, idx], ivf[idx] = f.cpu().numpy(), fl.cpu().numpy()
-        out = out + (tuple(iv[i].reshape(shape3) for i in range(3)) + (ivf.reshape(shape3),),)
-    if bootstrap is not None:                      # compact (k, t2, sigma) of the fit; the noise keyed by the flat index
-        args = (fit, fit_params, TEeffs, prior, norm, solver, kw.get("init_mode", "auto"), kw.get("max_iter", 0),
-                kw.get("tol", 0.0))
-        sg = (lambda a: a) if fit != "gaussian" else (lambda a: None)
-        if stream is not None:
-            bs = _bootstrap_pass(lib, p, *args, [maps[1][idx], maps[0][idx], sg(maps[2][idx])], None, None, bootstrap, 0.95,
-                                 0, None)
-            new = lambda t: torch.zeros(n_vox, dtype=t.dtype, device=y.device).index_copy_(0, idx, t)
-        else:
-            import torch
-            ps, (_, k, t2, s) = _staged(p, y[idx], maps[1][idx], maps[0][idx], sg(maps[2][idx]))
-            bs = _bootstrap_pass(lib, ps, *args, [k, t2, s], None, torch.from_numpy(idx).to(k.device), bootstrap, 0.95, 0,
-                                 None)
-
-            def new(t):
-                a = np.zeros(n_vox, dtype=t.cpu().numpy().dtype)
-                a[idx] = t.cpu().numpy()
-                return a
-        mean, sd, lo, hi, nu, no = bs
-        cols = (mean[1], sd[1], lo, hi, sd[0], sd[2] if fit != "gaussian" else torch.zeros_like(sd[2]), nu, no)
-        out = out + (BootstrapMaps(*[new(c).reshape(shape3) for c in cols]),)
+        f, fl, _ = _interval_pass(lib, ps, q, 64, False)
+        f = put(f)
+        out = out + (tuple(f[i].reshape(shape3) for i in range(3)) + (put(fl).reshape(shape3),),)
+    if bootstrap is not None:                      # the noise keyed by the flat voxel index
+        vid = torch.from_numpy(idx).to(k.device) if stream is None else None
+        mean, sd, lo, hi, nu, no = _bootstrap_pass(
+            lib, ps, fit, fit_params, TEeffs, prior, norm, solver, kw.get("init_mode", "auto"), kw.get("max_iter", 0),
+            kw.get("tol", 0.0), [k, t2, sg if fit != "gaussian" else None], None, vid, bootstrap, 0.95, 0, None)
+        if fit == "gaussian":
+            sd[2].zero_()
+        out = out + (BootstrapMaps(*[put(c).reshape(shape3) for c in (mean[1], sd[1], lo, hi, sd[0], sd[2], nu, no)]),)
     return out
 
 
@@ -758,15 +783,9 @@ def t2_interval(reshaped_t2w, mask_indices, TEeffs, fit, fit_params, prior=True,
     if not 16 <= int(n_grid) <= 256:
         raise ValueError("n_grid must lie in 16..256")
     t_lo, t_hi = (NO_PRIOR_T2_BOUNDS if not prior else (p.lb[1], p.ub[1]))
-    if _is_torch(reshaped_t2w):
-        keep += [_device_rows(p, reshaped_t2w, mask_indices)]
-        f, fl, pr = _interval_pass(lib, p, q, n_grid, False, profile, reshaped_t2w.device)
-    else:
-        y = np.asarray(reshaped_t2w)
-        if y.ndim != 2 or y.shape[1] != p.n_echo:
-            raise ValueError(f"reshaped_t2w must be [N, {p.n_echo}]")
-        ps, (ys,) = _staged(p, y if mask_indices is None else y[np.asarray(mask_indices)])
-        f, fl, pr = (t.cpu().numpy() if t is not None else None for t in _interval_pass(lib, ps, q, n_grid, True, profile, ys.device))
+    ps, _, _, fin, pin = _pass_input(p, reshaped_t2w, mask_indices)
+    keep += pin
+    f, fl, pr = (fin(t) for t in _interval_pass(lib, ps, q, n_grid, profile))
     lo, hi, best = f[0], f[1], f[2]
     del keep
     if not profile:
@@ -894,27 +913,10 @@ def parametric_bootstrap(reshaped_t2w, mask_indices, TEeffs, fit, fit_params, pr
         params = (r.k, r.t2, r.sigma if fit != "gaussian" else None)
     if len(params) != 3:
         raise ValueError("params must be (k, t2, sigma)")
-    dev_in = _is_torch(reshaped_t2w)
-    if dev_in:
-        keep += [_device_rows(p, reshaped_t2w, mask_indices)]
-        device = reshaped_t2w.device
-        vid, q = None, p
-        to_dev = lambda a: (a if _is_torch(a) else torch.from_numpy(np.ascontiguousarray(a))).to(
-            device=device, dtype=torch.float32).reshape(-1).contiguous()
-        par = [to_dev(a) if a is not None else None for a in params]
-    else:
-        y = np.asarray(reshaped_t2w)
-        if y.ndim != 2 or y.shape[1] != p.n_echo:
-            raise ValueError(f"reshaped_t2w must be [N, {p.n_echo}]")
-        ids = np.arange(y.shape[0], dtype=np.int64) if mask_indices is None else np.asarray(mask_indices).astype(np.int64)
-        if ids.size and (ids.min() < 0 or ids.max() >= y.shape[0]):
-            raise IndexError("mask_indices out of range")
-        host = lambda a: np.asarray(a.cpu() if _is_torch(a) else a)
-        q, (ys, *par) = _staged(p, y[ids], *[host(a) if a is not None else None for a in params])
-        device = ys.device
-        vid = torch.from_numpy(ids).to(device)
-        keep += [ys]
-        to_dev = lambda a: torch.from_numpy(np.ascontiguousarray(a, dtype=np.float32).reshape(-1)).to(device)
+    scalar_noise = noise_sd is not None and np.ndim(noise_sd) == 0 and not _is_torch(noise_sd)
+    q, (*par, noise), ids, fin, pin = _pass_input(p, reshaped_t2w, mask_indices, *params,
+                                                  None if scalar_noise else noise_sd)
+    keep += pin
     M = q.n_fit
     if fit == "gaussian":
         par[2] = None
@@ -922,21 +924,16 @@ def parametric_bootstrap(reshaped_t2w, mask_indices, TEeffs, fit, fit_params, pr
         raise ValueError(f"fit {fit!r} needs sigma in params")
     if any(a is not None and a.numel() != M for a in par):
         raise ValueError(f"params must hold {M} values each")
-    noise = None
-    if noise_sd is not None:
-        if np.ndim(noise_sd) == 0 and not _is_torch(noise_sd):
-            noise = torch.full((M,), float(noise_sd), dtype=torch.float32, device=device)
-        else:
-            noise = to_dev(noise_sd.cpu().numpy() if (_is_torch(noise_sd) and not dev_in) else noise_sd)
-            if noise.numel() != M:
-                raise ValueError(f"noise_sd must be a float or hold {M} values")
+    dev = torch.device("cuda", _state["device"])
+    if scalar_noise:
+        noise = torch.full((M,), float(noise_sd), dtype=torch.float32, device=dev)
+    elif noise is not None and noise.numel() != M:
+        raise ValueError(f"noise_sd must be a float or hold {M} values")
+    vid = torch.from_numpy(ids).to(dev) if ids is not None else None
     res = _bootstrap_pass(lib, q, fit, fit_params, TEeffs, prior, norm, solver, init_mode, 0, 0.0, par, noise, vid, n_rep,
                           level, seed, chunk)
     del keep
     P = 2 if fit == "gaussian" else 3
     mean, sd, lo, hi, nu, no = res
     mean, sd = mean[:P].t().contiguous(), sd[:P].t().contiguous()
-    out = (mean, sd, lo, hi, nu, no)
-    if not dev_in:
-        out = tuple(t.cpu().numpy() for t in out)
-    return BootstrapResult(*out)
+    return BootstrapResult(*(fin(t) for t in (mean, sd, lo, hi, nu, no)))

@@ -19,7 +19,7 @@
 //                 values; NaN with fewer than 2 used.  Sums run in a fixed order (kStatThreads partial sums, then a halving
 //                 tree), so the result does not depend on anything but the replicate values.
 //
-// Plain C++ when T2FIT_HOSTSIM is defined (tests/hostsim/bootstrap_shim.cpp checks it against oracle/bootstrap_oracle.py).
+// Plain C++ when T2FIT_HOSTSIM is defined (tests/hostsim/pass_shim.cpp checks it against oracle/bootstrap_oracle.py).
 #pragma once
 #include "../../include/t2fit.h"
 #include "t2fit_lbfgsb.cuh"

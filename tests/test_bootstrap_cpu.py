@@ -5,7 +5,7 @@ import pytest
 
 from oracle import bootstrap_oracle as bo
 from tests.conftest import load_golden
-from tests.hostsim import bootstrap_shim
+from tests.hostsim import pass_shim as bootstrap_shim
 
 FIXTURES = ["c1_gaussian_noprior", "c2_gaussian_hf_prior", "c3_floor_prior", "c3_rician_prior", "norm_gaussian",
             "cli3_gaussian_lf_noprior", "cli3_floor_hf_prior", "cli3_rician_hf_prior", "cli3_rician_lf_noprior",

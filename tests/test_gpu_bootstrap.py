@@ -10,7 +10,7 @@ import pytest
 from oracle import bootstrap_oracle as bo
 from oracle.fit_oracle import model_floor, model_mono
 from tests.conftest import fit_params_of, load_golden
-from tests.hostsim import bootstrap_shim
+from tests.hostsim import pass_shim as bootstrap_shim
 
 pytestmark = pytest.mark.gpu
 

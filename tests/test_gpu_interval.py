@@ -194,3 +194,18 @@ def test_empty_call_and_argument_errors(gpu_lib):
     assert call(p) == 0                                   # sigma bounds do not matter for 2 parameters
     assert call(problem(echoes=None)) == -1
     torch.cuda.synchronize()
+    # an index outside [0, N): host input raises what the fit raises, device input gives an invalid (NaN, flag 8) slot
+    fp = gpu_lib.preset("gaussian_rician", True)[1]
+    rows = np.abs(np.random.default_rng(0).normal(100.0, 10.0, (8, 4))).astype(np.float32)
+    par = (np.full(1, 600.0), np.full(1, 50.0), np.full(1, 5.0))
+    for bad in ([-1], [8]):
+        with pytest.raises(IndexError, match="mask_indices out of range"):
+            gpu_lib.t2_interval(rows, np.array(bad), te, "gaussian_rician", fp)
+        with pytest.raises(IndexError, match="mask_indices out of range"):
+            gpu_lib.parametric_bootstrap(rows, np.array(bad), te, "gaussian_rician", fp, n_rep=16, params=par)
+        with pytest.raises(IndexError, match="mask_indices out of range"):
+            gpu_lib.fit_voxels_batch(rows, np.array(bad), te, "gaussian_rician", fp, want=("se",))
+        lo, hi, best, fl = gpu_lib.t2_interval(torch.from_numpy(rows).cuda(), torch.tensor(bad, device="cuda"), te,
+                                               "gaussian_rician", fp)
+        torch.cuda.synchronize()
+        assert all(np.isnan(_np(a)).all() for a in (lo, hi, best)) and _np(fl).tolist() == [8], bad

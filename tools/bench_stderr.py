@@ -16,7 +16,6 @@ import argparse
 import ctypes as C
 import json
 import os
-import subprocess
 import sys
 
 import numpy as np
@@ -24,8 +23,10 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tools"))
 import fetal_t2mapping_b200 as t2                                      # noqa: E402
 from fetal_t2mapping_b200 import _abi, api, presets, synth             # noqa: E402
+from bench_interval import Flush, card, time_pass                      # noqa: E402
 
 HBM_PEAK = 7.7e12          # B/s, NVIDIA HGX B200 data sheet, one GPU
 FP64_PEAK = 37e12          # FLOP/s FP64, the same data sheet (296 TFLOP/s for eight GPUs)
@@ -42,35 +43,6 @@ WORK = {"gaussian": dict(flop=12, div=1, sqrt=0, exp=1, P=2),
 # per voxel after the echo loop: scaled Cholesky of a 2x2 / 3x3 matrix and the diagonal of its inverse
 FIXED = {2: dict(flop=12, div=4, sqrt=4), 3: dict(flop=40, div=8, sqrt=6)}
 CALL_FLOP = {"div": 10, "sqrt": 10, "exp": 20}          # FP64 instruction-equivalents of one call, for the FP64 roofline
-
-
-def card():
-    q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm", "--format=csv,noheader"],
-                       capture_output=True, text=True)
-    return q.stdout.strip().splitlines()[0] if q.returncode == 0 and q.stdout.strip() else torch.cuda.get_device_name(0)
-
-
-class Flush:
-    def __init__(self, dev):
-        self.buf = torch.empty(1 << 29, dtype=torch.uint8, device=dev)
-
-    def __call__(self):
-        self.buf.fill_(1)
-
-
-def time_pass(fn, flush, reps):
-    fn()
-    torch.cuda.synchronize()
-    ts = []
-    for _ in range(reps):
-        flush()
-        a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        a.record()
-        fn()
-        b.record()
-        b.synchronize()
-        ts.append(a.elapsed_time(b) * 1e3)
-    return float(np.median(ts)), [round(t, 1) for t in ts]
 
 
 def run_config(name, lib, flush, reps_fit, reps_se):
